@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config NAME] [--samples S]
                     [--impl ours|reference] [--no-cpu-baseline] [--no-reference-gpu] [--strong]
+                    [--dump-outputs DIR]
 
 Configurations (BASELINE.json `configs`, SURVEY.md 8(d)); `power_scan` is the headline and the default:
   power_scan  configs[1]: L=128, Length=2000 nm, T=80000 steps of 0.025 ns, 3 Power_scan excitations,
@@ -19,6 +20,12 @@ configurations are this step repeated.  Under torchrun every rank owns its own S
 the only exchange -- all-gather of lnL + global log-sum-exp over NCCL -- happens ONCE, after the last
 step, inside the timed region.  `strong` (N>1 or --strong) times one more step with a fixed global batch
 of 8 x S samples split over the ranks.
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller: lnl.npy (the likelihood table
+[E, S * ranks], float64), status.npy (per-sample solver status, float32) and, on more than one rank,
+lse.npy (the global log-sum-exp of the first file's lnL, float64).  Inputs are seeded, so two
+builds run with the same arguments can be compared output for output; the default batch S follows the
+kernel's occupancy, so give --samples when the two builds may differ in occupancy.
 
 `--impl reference` times the reference's own wired-in CPU path (bayeslib.simulate with has_GPU=False ->
 pvSim_fallback.pvSim_cpu_fallback, SciPy BDF; parallel_bayes_gpu.py:157-163) from baseline/_ref, one
@@ -42,6 +49,8 @@ TOL, MAXIT = 7, 10000
 METRIC = "param-sample likelihoods/sec (3-curve power scan)"
 UNIT = "likelihoods/s"
 FLOP_STEP, FLOP_ITER = 29, 126          # per node: per time step / per Newton iteration (SURVEY App. B)
+DUMP_BYTES = 60 * 2 ** 20               # cap of --dump-outputs: below 64 MB with the .npy headers
+DUMP_NAMES = ("lnl", "status", "lse", "sample_index")
 
 
 # ------------------------------------------------------------------------------------------------
@@ -137,6 +146,26 @@ class ClockSampler(threading.Thread):
         return {"sm_mhz": sm[len(sm) // 2], "sm_max_mhz": float(self.rows[0][1]),
                 "power_w_max": max(float(r[2]) for r in self.rows), "samples": len(self.rows),
                 "reasons": reasons}
+
+
+def dump_outputs(out_dir, per_sample, whole=None):
+    """Write host arrays as out_dir/<name>.npy: `per_sample` ones (last axis = parameter sample) and
+    `whole` ones (small, written as they are).  Above DUMP_BYTES a fixed, seeded subset of samples is
+    kept; its indices go to sample_index.npy.  Dump files of an earlier run that this run does not
+    write are removed, so the directory always holds one run's outputs."""
+    n = next(iter(per_sample.values())).shape[-1]
+    per_row = sum(a.itemsize * (a.size // n) for a in per_sample.values())
+    if per_row * n > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // (per_row + 8), replace=False))
+        per_sample = {name: a[..., keep] for name, a in per_sample.items()}
+        per_sample["sample_index"] = keep.astype(np.float64)
+    arrays = dict(per_sample, **(whole or {}))
+    os.makedirs(out_dir, exist_ok=True)
+    for name in DUMP_NAMES:
+        if name not in arrays and os.path.exists(os.path.join(out_dir, name + ".npy")):
+            os.remove(os.path.join(out_dir, name + ".npy"))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def host_threads():
@@ -297,7 +326,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-reference-gpu", action="store_true")
     ap.add_argument("--strong", action="store_true", help="also time one step of a fixed global batch (8 x S samples) split over the ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's lnL table and status as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours; the reference leg only times its CPU path")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -335,14 +369,15 @@ def main():
     lnl_steps = torch.zeros((args.steps, E, S), dtype=torch.float64, device=dev)     # every step's table, exchanged once
 
     def exchange(tables):
-        """The path's only exchange (SURVEY 8e): all-gather of per-sample lnL + global log-sum-exp."""
+        """The path's only exchange (SURVEY 8e): all-gather of per-sample lnL + global log-sum-exp.
+        Returns (gathered tables, log-sum-exp of the last table's first file, or None on one rank)."""
         if world == 1:
-            return tables
+            return tables, None
         flat = tables.reshape(-1, S)
         parts = [torch.empty_like(flat) for _ in range(world)]
         dist.all_gather(parts, flat)
-        D.global_logsumexp(trpl.engine.lse_partial(tables[-1, 0].contiguous()))
-        return torch.cat(parts, dim=-1)
+        lse = D.global_logsumexp(trpl.engine.lse_partial(tables[-1, 0].contiguous()))
+        return torch.cat(parts, dim=-1), lse
 
     def barrier():
         if world > 1:
@@ -371,10 +406,10 @@ def main():
         l2_flush.zero_()
         k0, k1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         k0.record()
-        trpl.engine.solve_loglik(Xd, problem, lnl=lnl_steps[k])
+        _, status_last, _ = trpl.engine.solve_loglik(Xd, problem, lnl=lnl_steps[k])
         k1.record()
         kern_ev.append((k0, k1))
-    exchange(lnl_steps)
+    tables, lse = exchange(lnl_steps)
     ev1.record()
     barrier()
     ms_total = ev0.elapsed_time(ev1)
@@ -499,6 +534,16 @@ def main():
         if world == 1 and not args.no_cpu_baseline:
             out["cpu_baseline"] = cpu_baselines(cfg, args.config, host_threads())
         print(json.dumps(out))
+    if args.dump_outputs:
+        lnl_last = tables.reshape(-1, tables.shape[-1])[-E:]          # [E, S * world]: last step, all ranks
+        if world > 1:
+            parts = [torch.empty_like(status_last) for _ in range(world)]
+            dist.all_gather(parts, status_last)
+            status_last = torch.cat(parts)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"lnl": lnl_last.cpu().numpy(),
+                                             "status": status_last.cpu().numpy().astype(np.float32)},
+                         {} if lse is None else {"lse": lse.cpu().numpy()})
     if world > 1:
         dist.destroy_process_group()
 

@@ -2,8 +2,8 @@
 `probs.py`, `bayeslib.bayes`), SURVEY 8(c) "exact oracle, GPU box".
 
 Two sources for the reference side:
-  * live: `baseline/_ref/` (git-ignored copy of the reference that ships to the GPU box with the
-    snapshot) is imported and run on the same GPU, same inputs, inside the test;
+  * live: `baseline/_ref/` (a git-ignored copy of the reference's source, when present) is imported
+    and run on the same GPU, same inputs, inside the test;
   * committed fixtures `tests/golden/ref_b200_*.npz`: outputs of that same code on a B200, written by
     `tools/ref_on_b200.py` (16 samples x 3 curves of the full T=80000 PL curves sub-sampled in time;
     the 256-sample likelihood table of the reference's `bayeslib.bayes`).
@@ -114,28 +114,59 @@ def test_bayes_matches_native_reference_golden():
 
 
 # ------------------------------------------------------------------------------------------------
-# GPU, live: the reference itself on this GPU (skipped when baseline/_ref did not travel)
+# GPU, live: the reference itself on this GPU, when its source is in baseline/_ref
 # ------------------------------------------------------------------------------------------------
 def _live_reference():
+    """(baseline.ref_runner, None) when the reference's source is in baseline/_ref and numba can run
+    it on the GPU, else (None, the reason it cannot)."""
     sys.path.insert(0, ROOT)
     from baseline import ref_runner as rr
     if not rr.available():
-        pytest.skip("baseline/_ref (copy of the reference) is not present on this box")
+        return None, "baseline/_ref (copy of the reference's source) is not present"
     try:
         from numba import cuda
         if not cuda.is_available():
-            pytest.skip("numba sees no CUDA device")
+            return None, "numba sees no CUDA device"
     except Exception as e:                                  # pragma: no cover
-        pytest.skip("numba.cuda unusable: %r" % (e,))
-    return rr
+        return None, "numba.cuda unusable: %r" % (e,)
+    return rr, None
+
+
+def _check_pl_and_lnl(pl, ref, X, simPar, what):
+    """PL criterion, then the likelihood of every sample whose curve stays clear of the cancellation
+    floor, evaluated the same way on both sides (f64 log10, residual against the reference curve of
+    the truth sample, row 0)."""
+    floor = pl_noise_floor(X[:, :12], simPar[0], simPar[1], simPar[2], simPar[3])
+    ex = _pl_excess(pl, ref, floor)
+    assert ex.max() <= 1.0, "%s: worst excess %.3g" % (what, ex.max())
+    clean = (np.abs(ref) > 1e6 * floor[:, None]).all(axis=1)
+    assert clean.mean() > 0.5
+    lr, lm = np.log10(ref[clean]), np.log10(pl[clean])
+    tgt = np.log10(ref[0])
+    l_ref = -((lr - tgt) ** 2).sum(axis=1)
+    l_my = -((lm - tgt) ** 2).sum(axis=1)
+    np.testing.assert_allclose(l_my[1:], l_ref[1:], rtol=1e-6)
 
 
 @pytest.mark.gpu
 def test_pvsim_matches_reference_numba_kernels_live():
-    """pvSimPCR.pvSim (numba-CUDA, unmodified, float64 PL buffer) vs trpl.pvSim on the same 384 prior
-    samples: highest-power curve at the full T=80000, the two others over the first 8000 steps."""
+    """pvSimPCR.pvSim (numba-CUDA, unmodified, float64 PL buffer) vs trpl.pvSim.  Live: the same 384
+    prior samples, highest-power curve at the full T=80000, the two others over the first 8000 steps.
+    Without the reference's source: its stored B200 output (16 prior samples, all 3 curves at the full
+    T=80000, 578 time points; tests/golden/ref_b200_pvsim.npz)."""
     import bayesian_inference_trpl_b200 as trpl
-    rr = _live_reference()
+    rr, _ = _live_reference()
+    if rr is None:
+        g, simPar = _golden_case()
+        X = g["X"]
+        for c in range(3):
+            pl = np.empty((len(X), simPar[3] + 1))
+            st = np.zeros(len(X), dtype=np.int32)
+            trpl.pvSim(pl, None, None, None, X[:, :12], simPar, g["inis"][c], (128,), 0, 1, init_mode="points",
+                       status_out=st)
+            assert (st == 0).all()
+            _check_pl_and_lnl(pl[:, g["t_idx"]], g["pl_ref_c%d" % c], X, simPar, "stored curve %d" % c)
+        return
     inis = power_scan_excitations()
     S = 384
     X = prior_samples(S, seed=77)
@@ -147,28 +178,20 @@ def test_pvsim_matches_reference_numba_kernels_live():
         st = np.zeros(S, dtype=np.int32)
         trpl.pvSim(pl, None, None, None, X[:, :12], simPar, inis[c], (128,), 0, 1, init_mode="points", status_out=st)
         assert (st == 0).all() and np.isfinite(ref).all()
-        floor = pl_noise_floor(X[:, :12], 2000.0, simPar[1], 128, T)
-        ex = _pl_excess(pl, ref, floor)
-        assert ex.max() <= 1.0, "curve %d: worst excess %.3g" % (c, ex.max())
-        # likelihood of every sample whose curve stays clear of the cancellation floor, evaluated the
-        # same way on both sides (f64 log10, residual against the truth sample's reference curve)
-        clean = (np.abs(ref) > 1e6 * floor[:, None]).all(axis=1)
-        assert clean.mean() > 0.5
-        lr, lm = np.log10(ref[clean]), np.log10(pl[clean])
-        tgt = np.log10(ref[0])
-        l_ref = -((lr - tgt) ** 2).sum(axis=1)
-        l_my = -((lm - tgt) ** 2).sum(axis=1)
-        np.testing.assert_allclose(l_my[1:], l_ref[1:], rtol=1e-6)
+        _check_pl_and_lnl(pl, ref, X, simPar, "curve %d" % c)
 
 
 @pytest.mark.gpu
 def test_reference_bayeslib_drives_the_dropins_live():
     """INTEGRATION.md route A: the reference's own, unmodified bayeslib.bayes with
     sys.modules["probs"] = trpl.probs and model = trpl.pvSim reproduces the likelihood table of the
-    all-reference run (its numba solver, fastlog and prob kernels) on the same GPU."""
+    all-reference run (its numba solver, fastlog and prob kernels) on the same GPU.  What it checks is
+    that unmodified source driving the drop-ins, so it needs that source in baseline/_ref."""
     import bayesian_inference_trpl_b200 as trpl
     from oracle import oracle
-    rr = _live_reference()
+    rr, why = _live_reference()
+    if rr is None:
+        pytest.skip(why)
     inis = power_scan_excitations()
     T = 2000
     case = route_a_case(inis, 96, T, truth_pl=lambda c: oracle.solve(
