@@ -14,24 +14,13 @@ namespace trpl {
 
 
 constexpr unsigned FULL = 0xffffffffu;
-constexpr int WARPS_PER_CTA = 4;
-#ifndef TRPL_MIN_CTAS
-#define TRPL_MIN_CTAS 4
-#endif
-// A/B switches of the solver (defaults = the shipped configuration; profiles/r02_variants.txt)
-#ifndef TRPL_MINOR_PIVOTS
-#define TRPL_MINOR_PIVOTS 0        // 1: pivot reciprocals from leading minors (independent, 3 more DMUL)
-#endif
-#ifndef TRPL_CTA_LAT
-#define TRPL_CTA_LAT 1             // multi-warp simulations: pivots from leading minors (independent reciprocals)
-#endif
-#ifndef TRPL_CONST_TABLE
-#define TRPL_CONST_TABLE 1         // 1: derived per-simulation constants parked in lanes and read by shuffles
-#endif
-#ifndef TRPL_PCR_LAST_EXP
-#define TRPL_PCR_LAST_EXP 35       // off-diagonals below 2^-this: the PCR stage degenerates to a B-only update
-#endif
+constexpr int WARPS_PER_CTA = 4;      // warp kernel: one simulation per warp
+constexpr int MIN_CTAS_PER_SM = 4;    // its __launch_bounds__ occupancy target (16 warps per SM)
 
+// The solver's design choices (pivot scheme per kernel family, constant table, B-only last PCR stage)
+// are fixed in the code; the measurements behind them are in profiles/r02_variants.txt.  The only
+// build flag that selects other code is TRPL_DEBUG.
+//
 // -DTRPL_DEBUG=1: the sanitizer substitute (compute-sanitizer is closed on the pool this was developed on):
 // device-side bounds checks on every ring slot, observation index and exchange-buffer row, and a canary
 // word behind each warp's ring that is verified after every simulation.  A violation prints the site and

@@ -135,8 +135,16 @@ void cfg_shape(const Cfg &c, int *threads, int *sims_per_cta, size_t *smem)
     }
 }
 
-int kernel_geometry(int device, const Cfg &cfg, kern_t *k_out, size_t *smem_out, int *ctas_per_sm,
-                    int *sms)
+// Launch geometry of a configuration on `device`: kernel, threads and simulations per CTA, dynamic shared
+// memory, resident CTAs per SM and SM count.
+struct Geometry {
+    kern_t k;
+    int threads, sims_per_cta;
+    size_t smem;
+    int ctas_per_sm, sms;
+};
+
+int kernel_geometry(int device, const Cfg &cfg, Geometry *geo)
 {
     kern_t k = pick_kernel(cfg);
     int threads, spc; size_t smem;
@@ -148,8 +156,28 @@ int kernel_geometry(int device, const Cfg &cfg, kern_t *k_out, size_t *smem_out,
     if (nb < 1) return TRPL_EUNSUPPORTED;
     int nsm = 0;
     CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
-    *k_out = k; *smem_out = smem; *ctas_per_sm = nb; *sms = nsm;
+    *geo = Geometry{k, threads, spc, smem, nb, nsm};
     return TRPL_OK;
+}
+
+// KArgs fields shared by both entry points: tolerance 10^-tol, BDF order clamped to 1..5 (out of range = 5)
+void init_kargs(KArgs &ka, int L, int tol, int max_iter, int max_order)
+{
+    memset(&ka, 0, sizeof(ka));
+    ka.TOL = pow(10.0, -(double)tol);
+    ka.L = L;
+    ka.max_iter = max_iter;
+    ka.max_order = (max_order < 1 || max_order > 5) ? 5 : max_order;
+}
+
+// scales, initial-profile factor and PL re-dimensioning of one curve (pvSimPCR.py:327-331, :393)
+void init_curve(CurveDev &cv, double length, double time, int L, int T, int flags, const double *d_init)
+{
+    double dx, dt;
+    make_scales(length, time, L, T, cv.scales, &dx, &dt);
+    cv.init_mul = (flags & TRPL_F_INIT_GRID_UNITS) ? 1.0 : cv.scales[0];
+    cv.redim = pow(dx, 2.0) * dt;
+    cv.init = d_init;
 }
 
 // Makes `device` current for the duration of one C-ABI call and restores the caller's device on every
@@ -176,8 +204,8 @@ struct DeviceGuard {
 
 int launch_sims(KArgs &ka, const Cfg &cfg, int device, cudaStream_t st)
 {
-    kern_t k; size_t smem; int nb, nsm;
-    int rc = kernel_geometry(device, cfg, &k, &smem, &nb, &nsm);
+    Geometry geo;
+    int rc = kernel_geometry(device, cfg, &geo);
     if (rc) return rc;
     // longest-processing-time-first order of the curves (insertion sort, C <= 8)
     for (int c = 0; c < ka.C; c++) ka.curve_order[c] = c;
@@ -189,14 +217,12 @@ int launch_sims(KArgs &ka, const Cfg &cfg, int device, cudaStream_t st)
     CK(counter.alloc(sizeof(unsigned long long)));
     CK(cudaMemsetAsync(counter.p, 0, sizeof(unsigned long long), st));
     ka.counter = (unsigned long long *)counter.p;
-    int threads, spc; size_t smem2;
-    cfg_shape(cfg, &threads, &spc, &smem2);
     const unsigned long long items = (unsigned long long)ka.S * ka.C;
-    unsigned long long want = (items + spc - 1) / spc;
-    unsigned long long cap = (unsigned long long)nb * nsm;
+    unsigned long long want = (items + geo.sims_per_cta - 1) / geo.sims_per_cta;
+    unsigned long long cap = (unsigned long long)geo.ctas_per_sm * geo.sms;
     const unsigned grid = (unsigned)(want < cap ? want : cap);
     if (grid > 0) {
-        k<<<grid, threads, smem, st>>>(ka);
+        geo.k<<<grid, geo.threads, geo.smem, st>>>(ka);
         CK(cudaGetLastError());
     }
     return TRPL_OK;
@@ -233,12 +259,10 @@ int trpl_resident_sims(int device, int L)
     DeviceGuard guard;
     rc = guard.enter(device);
     if (rc) return rc;
-    kern_t k; size_t smem; int nb, nsm;
-    rc = kernel_geometry(device, cfg, &k, &smem, &nb, &nsm);
+    Geometry geo;
+    rc = kernel_geometry(device, cfg, &geo);
     if (rc) return rc;
-    int threads, spc; size_t smem2;
-    cfg_shape(cfg, &threads, &spc, &smem2);
-    return nb * nsm * spc;
+    return geo.ctas_per_sm * geo.sms * geo.sims_per_cta;
 }
 
 int trpl_solve_pl(const double *d_matpar, int64_t S, int64_t ld_matpar, const double *d_init,
@@ -258,23 +282,16 @@ int trpl_solve_pl(const double *d_matpar, int64_t S, int64_t ld_matpar, const do
     if (rc) return rc;
     if (S == 0) return TRPL_OK;
     cudaStream_t st = (cudaStream_t)stream;
-    if (max_order < 1 || max_order > 5) max_order = 5;
 
     KArgs ka;
-    memset(&ka, 0, sizeof(ka));
+    init_kargs(ka, L, tol, max_iter, max_order);
     ka.x = d_matpar; ka.ldx = ld_matpar; ka.S = S; ka.pl_stride = pl_stride;
-    ka.TOL = pow(10.0, -(double)tol);
     ka.sse = nullptr; ka.status = d_status; ka.iters = (long long *)d_iters;
-    ka.mag_col = -1; ka.C = 1; ka.E = 0; ka.L = L; ka.plT = plT; ka.max_iter = max_iter;
-    ka.max_order = max_order;
+    ka.mag_col = -1; ka.C = 1; ka.E = 0; ka.plT = plT;
     ka.flags = (flags & TRPL_F_INIT_GRID_UNITS) | (pl_dtype == TRPL_F32 ? TRPL_F_EMULATE_F32 : 0);
     ka.pl_dtype = pl_dtype;
     CurveDev &cv = ka.curves[0];
-    double dx, dt;
-    make_scales(length, time, L, T, cv.scales, &dx, &dt);
-    cv.init_mul = (flags & TRPL_F_INIT_GRID_UNITS) ? 1.0 : cv.scales[0];
-    cv.redim = pow(dx, 2.0) * dt;
-    cv.init = d_init;
+    init_curve(cv, length, time, L, T, flags, d_init);
     cv.pl_out = d_pl;
     cv.t_last = T;
     return launch_sims(ka, cfg, device, st);
@@ -297,24 +314,18 @@ int trpl_solve_loglik(const double *d_x, int64_t S, int64_t ldx, int mag_col,
     if (rc) return rc;
     if (S == 0) return TRPL_OK;
     cudaStream_t st = (cudaStream_t)stream;
-    if (max_order < 1 || max_order > 5) max_order = 5;
 
     KArgs ka;
-    memset(&ka, 0, sizeof(ka));
+    init_kargs(ka, L, tol, max_iter, max_order);
     ka.x = d_x; ka.ldx = ldx; ka.S = S; ka.pl_stride = 0;
-    ka.TOL = pow(10.0, -(double)tol);
     ka.sse = d_sse; ka.iters = (long long *)d_iters;
-    ka.mag_col = mag_col; ka.C = C; ka.E = E; ka.L = L; ka.plT = 1; ka.max_iter = max_iter;
-    ka.max_order = max_order; ka.flags = flags; ka.pl_dtype = TRPL_F64;
+    ka.mag_col = mag_col; ka.C = C; ka.E = E; ka.plT = 1;
+    ka.flags = flags; ka.pl_dtype = TRPL_F64;
     for (int c = 0; c < C; c++) {
         const trpl_curve &src = curves[c];
         if (!src.d_init || !(src.length > 0)) return TRPL_EINVAL;
         CurveDev &cv = ka.curves[c];
-        double dx, dt;
-        make_scales(src.length, time, L, T, cv.scales, &dx, &dt);
-        cv.init_mul = (flags & TRPL_F_INIT_GRID_UNITS) ? 1.0 : cv.scales[0];
-        cv.redim = pow(dx, 2.0) * dt;
-        cv.init = src.d_init;
+        init_curve(cv, src.length, time, L, T, flags, src.d_init);
         cv.pl_out = nullptr;
         cv.t_last = 0;
         for (int e = 0; e < E; e++) {

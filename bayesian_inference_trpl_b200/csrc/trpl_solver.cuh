@@ -1,8 +1,11 @@
 // trpl_solver.cuh -- the forward-model + fused-likelihood kernels (the hot path):
-// Comm<W> (lane communication policy), tridiag_solve, Ring, run_sim, trpl_sim_kernel<M,PAD>,
-// trpl_sim_cta_kernel<W,M,PADM>.  Replaces pvSimPCR.py:14-293 and bayeslib.py:150-196.
-// Lines tagged [sec:NAME] delimit the sections profiles/sass_budget.py attributes SASS instructions to.
+// Comm<W> (lane communication policy), tridiag_solve (partition_sweep, warp_solve, cta_solve), Ring,
+// run_sim, trpl_sim_kernel<M,PAD>, trpl_sim_cta_kernel<W,M,PADM>.  Replaces pvSimPCR.py:14-293 and
+// bayeslib.py:150-196.  Comment lines tagged "[sec:" + a section name + "]" delimit the sections that
+// profiles/sass_budget.py attributes SASS instructions to.
 #pragma once
+#include <type_traits>
+
 #include "trpl_common.cuh"
 
 namespace trpl {
@@ -40,6 +43,11 @@ struct Comm {
     static constexpr int SB_STRIDE = 32 + (W > 1 ? 16 / W : 0);
     static constexpr int SB_PLANE = SB_STRIDE * W;
     static __device__ __forceinline__ int slot(const int r) { return (r % W) * SB_STRIDE + r / W; }
+
+    // W > 1: `buf` holds xb, red and sb back to back; the solver role starts at warp `solver0`
+    __device__ __forceinline__ explicit Comm(const int g_, double *buf = nullptr, const int solver0 = 0)
+        : g(g_), xb(buf), red(W > 1 ? buf + 2 * XB_K * 32 * W : nullptr), phase(0), rphase(0),
+          sb(W > 1 ? red + 2 * W * 4 : nullptr), solver(solver0) {}
 
     // K values from lane g-dm (-> vm) and lane g+dp (-> vp); out-of-range sources return the
     // caller's own value (always multiplied by an exact zero downstream).  For W > 1 the barrier
@@ -164,33 +172,25 @@ __device__ __forceinline__ void pcr_stage(double &Lr, double &Ur, double &Br, co
 
 // Tridiagonal solve, M rows per lane (row n = M*g + j):  l[j] x[n-1] + d[j] x[n] + u[j] x[n+1] = b[j].
 // Rows outside the physical system must be identity rows (l=u=0, d=1).  l of the first row
-// and u of the last physical row must be 0.
-// Returns the new value of the previous lane's last node (needed by the callers anyway).
+// and u of the last physical row must be 0.  Every lane first eliminates its M-1 interior rows
+// (partition_sweep), which leaves one interface row per lane; the two kernel families then solve the
+// interface system in their own way (warp_solve, cta_solve).  Both return the new value of the previous
+// lane's last node (needed by the callers anyway) and store the new value of the NEXT lane's first node
+// in xr.
 //
-// W == 1: register-local partition sweep over the M-1 interior rows of every lane, then parallel cyclic
-// reduction over the 32 interface rows with warp shuffles.
-// W  > 1 (one CTA per simulation): the same lane-local sweep; the 32*W interface rows are then handed to
-// ONE warp through shared memory, which holds W of them per lane and solves them with the W == 1 code
-// (a second partition level + shuffle PCR): two block barriers per solve instead of one per PCR stage
-// over 32*W unknowns.  The solver role rotates over the warps from solve to solve: warp k of every CTA
-// sits on scheduler k, so a fixed solver warp would load one scheduler of the SM with the serial part
-// of all resident CTAs (+46 % time per iteration, measured).  The neighbour values the caller needs (previous lane's last node, next lane's
-// first node) are rebuilt from the interface solution, so no further exchange follows the solve.
-// xr receives the new value of the NEXT lane's first node.
-// LAT = latency-optimised variant (multi-warp simulations run 2 warps per scheduler, so dependent
-// chains are exposed): pivot reciprocals from the leading minors, which are independent of each other,
-// instead of the Thomas recurrence (3 multiplies fewer, but M-1 reciprocals in series).
-template <int M, int W, bool LAT = (W > 1) && (TRPL_CTA_LAT != 0)>
-__device__ __forceinline__ double tridiag_solve(const double (&l)[M], const double (&d)[M],
+// Pivots of the sweep, chosen per kernel family (each measured better on its own kernel,
+// profiles/r02_variants.txt): the warp kernel uses the Thomas recurrence (3 multiplies fewer, but M-1
+// reciprocals in series); the CTA kernel, whose simulations run 2 warps per scheduler and so expose
+// dependent chains, uses reciprocals of the leading minors, which are independent of each other.
+
+// [sec:partition] interior rows 0..M-2 of a lane (M > 1):  x_j = y_j - v_j * s_left - w_j * s_own
+template <int M, bool MINOR_PIVOTS>
+__device__ __forceinline__ void partition_sweep(const double (&l)[M], const double (&d)[M],
                                                 const double (&u)[M], const double (&b)[M],
-                                                double (&x)[M], Comm<W> &cm, double &xr)
+                                                double (&y)[M - 1], double (&v)[M - 1], double (&w)[M - 1])
 {
-    // [sec:partition]
-    double Lr, Dr, Ur, Br;
-    double c[M > 1 ? M - 1 : 1], y[M > 1 ? M - 1 : 1], v[M > 1 ? M - 1 : 1], w[M > 1 ? M - 1 : 1];
-    if constexpr (M > 1) {
-        // interior rows 0..M-2:  x_j = y_j - v_j * s_left - w_j * s_own
-        if constexpr (LAT || TRPL_MINOR_PIVOTS) {
+    double c[M - 1];
+    if constexpr (MINOR_PIVOTS) {
         // Pivot reciprocals from the leading principal minors m_{j+1} = d_j m_j - l_j u_{j-1} m_{j-1}
         // (1/pivot_j = m_j / m_{j+1}): independent reciprocals, 3 more multiplies per solve.
         double ip[M - 1];
@@ -213,7 +213,7 @@ __device__ __forceinline__ double tridiag_solve(const double (&l)[M], const doub
             y[j] = fma(-l[j], y[j - 1], b[j]) * ip[j];
             v[j] = (-l[j] * v[j - 1]) * ip[j];
         }
-        } else {
+    } else {
         // Thomas forward sweep: pivot_j = d_j - l_j c_{j-1}
         {
             const double ip0 = rcp64(d[0]);
@@ -228,95 +228,47 @@ __device__ __forceinline__ double tridiag_solve(const double (&l)[M], const doub
             y[j] = fma(-l[j], y[j - 1], b[j]) * ipj;
             v[j] = (-l[j] * v[j - 1]) * ipj;
         }
-        }
-        w[M - 2] = c[M - 2];
+    }
+    w[M - 2] = c[M - 2];
 #pragma unroll
-        for (int j = M - 3; j >= 0; j--) {
-            y[j] = fma(-c[j], y[j + 1], y[j]);
-            v[j] = fma(-c[j], v[j + 1], v[j]);
-            w[j] = -c[j] * w[j + 1];
-        }
-        if constexpr (W > 1) {
-            // Shared-memory planes (rows at Comm::slot): 0-6 = input of the solver warp, written by every
-            // lane before barrier 1 and read by warp 0 only; 7-8 = output (interface solution z, and the
-            // next lane's first node xr), written by warp 0 before barrier 2 and read by every lane after
-            // it.  Inputs and outputs never share a plane, so one buffer is enough: the next solve's
-            // inputs are written after barrier 2 of this one, its outputs after its own barrier 1.
-            constexpr int G = 32 * W, PL_ = Comm<W>::SB_PLANE, ST_ = Comm<W>::SB_STRIDE;
-            const int g = cm.g;
-            double *sb = cm.sb;
-            const int me = Comm<W>::slot(g);
-            TRPL_DASSERT(me >= 0 && me < PL_ && g < G);
-            const double lr = l[M - 1];
-            sb[0 * PL_ + me] = y[0];
-            sb[1 * PL_ + me] = v[0];
-            sb[2 * PL_ + me] = w[0];
-            sb[3 * PL_ + me] = -lr * v[M - 2];                      // this lane's share of its interface row
-            sb[4 * PL_ + me] = fma(-lr, w[M - 2], d[M - 1]);
-            sb[5 * PL_ + me] = fma(-lr, y[M - 2], b[M - 1]);
-            sb[6 * PL_ + me] = u[M - 1];
-            __syncthreads();
-            if ((g >> 5) == cm.solver) {
-                const int sl_ = g & 31;                            // solver lane: rows W*sl_ .. W*sl_+W-1
-                double L2[W], D2[W], U2[W], B2[W], Z[W];
-#pragma unroll
-                for (int k = 0; k < W; k++) {
-                    const int r = W * sl_ + k;                     // slot(r) = k * ST_ + sl_
-                    const int here = k * ST_ + sl_;
-                    const int next = (k + 1 < W) ? here + ST_ : ((sl_ < 31) ? sl_ + 1 : here);
-                    const double ur = (r < G - 1) ? sb[6 * PL_ + here] : 0.0;
-                    L2[k] = sb[3 * PL_ + here];
-                    D2[k] = fma(-ur, sb[1 * PL_ + next], sb[4 * PL_ + here]);
-                    U2[k] = -ur * sb[2 * PL_ + next];
-                    B2[k] = fma(-ur, sb[0 * PL_ + next], sb[5 * PL_ + here]);
-                }
-                Comm<1> c1;
-                c1.g = sl_; c1.xb = nullptr; c1.red = nullptr; c1.phase = 0; c1.rphase = 0; c1.sb = nullptr; c1.solver = 0;
-                double znext;                                      // first row of the next lane
-                tridiag_solve<W, 1, (TRPL_CTA_LAT != 0)>(L2, D2, U2, B2, Z, c1, znext);
-#pragma unroll
-                for (int k = 0; k < W; k++) {
-                    const int here = k * ST_ + sl_;
-                    const int next = (k + 1 < W) ? here + ST_ : ((sl_ < 31) ? sl_ + 1 : here);
-                    const double zn = (k + 1 < W) ? Z[k + 1] : znext;
-                    sb[7 * PL_ + here] = Z[k];
-                    sb[8 * PL_ + here] = fma(-sb[2 * PL_ + next], zn, fma(-sb[1 * PL_ + next], Z[k], sb[0 * PL_ + next]));
-                }
-            }
-            __syncthreads();
-            cm.solver = (cm.solver + 1) & (W - 1);     // the role rotates: every scheduler gets its share of the serial part
-            const double z = sb[7 * PL_ + me];
-            const double zl = (g > 0) ? sb[7 * PL_ + Comm<W>::slot(g - 1)] : 0.0;
-            xr = (g < G - 1) ? sb[8 * PL_ + me] : 0.0;
-            x[M - 1] = z;
-#pragma unroll
-            for (int j = 0; j < M - 1; j++) x[j] = fma(-w[j], z, fma(-v[j], zl, y[j]));
-            return zl;
-        }
-        if constexpr (W == 1) {
-            // interface row (local M-1) couples s_left, s_own and the next lane's first interior row
-            double mine[3] = {y[0], v[0], w[0]}, nm[3], nx[3];
-            cm.template xchg<3, false, true>(mine, 1, 1, nm, nx);
-            const double y0n = nx[0], v0n = nx[1], w0n = nx[2];
-            const double lr = l[M - 1], ur = u[M - 1];
-            Lr = -lr * v[M - 2];
-            Dr = fma(-ur, v0n, fma(-lr, w[M - 2], d[M - 1]));
-            Ur = -ur * w0n;
-            Br = fma(-ur, y0n, fma(-lr, y[M - 2], b[M - 1]));
-        }
+    for (int j = M - 3; j >= 0; j--) {
+        y[j] = fma(-c[j], y[j + 1], y[j]);
+        v[j] = fma(-c[j], v[j + 1], v[j]);
+        w[j] = -c[j] * w[j + 1];
+    }
+}
+
+// One warp, 32 interface rows (one per lane): parallel cyclic reduction with warp shuffles, then
+// back-substitution.  Used by the warp kernel and by the solver warp of the CTA kernel.
+template <int M, bool MINOR_PIVOTS>
+__device__ __forceinline__ double warp_solve(const double (&l)[M], const double (&d)[M], const double (&u)[M],
+                                             const double (&b)[M], double (&x)[M], Comm<1> &cm, double &xr)
+{
+    double Lr, Dr, Ur, Br;
+    double y[M > 1 ? M - 1 : 1], v[M > 1 ? M - 1 : 1], w[M > 1 ? M - 1 : 1];
+    if constexpr (M > 1) {
+        partition_sweep<M, MINOR_PIVOTS>(l, d, u, b, y, v, w);
+        // interface row (local M-1) couples s_left, s_own and the next lane's first interior row
+        double mine[3] = {y[0], v[0], w[0]}, nm[3], nx[3];
+        cm.xchg<3, false, true>(mine, 1, 1, nm, nx);
+        const double y0n = nx[0], v0n = nx[1], w0n = nx[2];
+        const double lr = l[M - 1], ur = u[M - 1];
+        Lr = -lr * v[M - 2];
+        Dr = fma(-ur, v0n, fma(-lr, w[M - 2], d[M - 1]));
+        Ur = -ur * w0n;
+        Br = fma(-ur, y0n, fma(-lr, y[M - 2], b[M - 1]));
     } else {
         Lr = l[0]; Dr = d[0]; Ur = u[0]; Br = b[0];
     }
-    static_assert(W == 1 || M > 1, "multi-warp simulations keep at least 2 nodes per lane");
-    if constexpr (W > 1) {
-        return 0.0;        // not reached: the multi-warp path returned above
-    } else {
-    // [sec:normalise] parallel cyclic reduction over the 32*W interface unknowns, unit diagonal
+    // [sec:normalise] parallel cyclic reduction over the 32 interface unknowns, unit diagonal
     {
         double inv = rcp64(Dr);
         Lr *= inv; Ur *= inv; Br *= inv;
     }
     // [sec:pcr]
+    // off-diagonals below 2^-PCR_LAST_EXP: the stage degenerates to a B-only update.  At 35 that is exact
+    // (see below); a 2^-27 threshold measured 1.3 % faster but is not bit-identical (profiles/r02_variants.txt).
+    constexpr int PCR_LAST_EXP = 35;
 #pragma unroll
     for (int rf = 1; rf < 32; rf <<= 1) {
         // Off-diagonals shrink quadratically per stage.  Let m = max |L|,|U| over the simulation:
@@ -328,17 +280,17 @@ __device__ __forceinline__ double tridiag_solve(const double (&l)[M], const doub
         // an initial one below 2^-9, i.e. practically no transport; those cases just run 3 stages.)
         const int hl = __double2hiint(Lr) & 0x7fffffff, hu = __double2hiint(Ur) & 0x7fffffff;
         const int hm = max(hl, hu);
-        const bool busy = (rf < 8) || (hm >= ((1023 - TRPL_PCR_LAST_EXP) << 20));
+        const bool busy = (rf < 8) || (hm >= ((1023 - PCR_LAST_EXP) << 20));
         if (rf >= 8 && !__any_sync(FULL, busy)) {
             if (__any_sync(FULL, hm >= ((1023 - 70) << 20))) {
                 double mine[1] = {Br}, vm[1], vp[1];
-                cm.template xchg<1, true, true>(mine, rf, rf, vm, vp);
+                cm.xchg<1, true, true>(mine, rf, rf, vm, vp);
                 Br = fma(-vp[0], Ur, fma(-vm[0], Lr, Br));
             }
             break;
         }
         double mine[3] = {Lr, Ur, Br}, vm[3], vp[3];
-        cm.template xchg<3, true, true>(mine, rf, rf, vm, vp);
+        cm.xchg<3, true, true>(mine, rf, rf, vm, vp);
         pcr_stage(Lr, Ur, Br, vm, vp);
     }
     // [sec:backsubst]
@@ -350,7 +302,85 @@ __device__ __forceinline__ double tridiag_solve(const double (&l)[M], const doub
     }
     xr = cm.from_next(x[0]);
     return sl;
-    }   // W == 1
+}
+
+// [sec:partition] One CTA of W warps, 32*W interface rows.  They are handed to ONE warp through shared
+// memory, which holds W of them per lane and solves them with warp_solve (a second partition level +
+// shuffle PCR): two block barriers per solve instead of one per PCR stage over 32*W unknowns.  The
+// solver role rotates over the warps from solve to solve: warp k of every CTA sits on scheduler k, so a
+// fixed solver warp would load one scheduler of the SM with the serial part of all resident CTAs (+46 %
+// time per iteration, measured).  The neighbour values the caller needs (previous lane's last node,
+// next lane's first node) are rebuilt from the interface solution, so no further exchange follows.
+template <int M, int W>
+__device__ __forceinline__ double cta_solve(const double (&l)[M], const double (&d)[M], const double (&u)[M],
+                                            const double (&b)[M], double (&x)[M], Comm<W> &cm, double &xr)
+{
+    static_assert(W > 1 && M > 1, "multi-warp simulations keep at least 2 nodes per lane");
+    double y[M - 1], v[M - 1], w[M - 1];
+    partition_sweep<M, true>(l, d, u, b, y, v, w);
+    // Shared-memory planes (rows at Comm::slot): 0-6 = input of the solver warp, written by every
+    // lane before barrier 1 and read by the solver warp only; 7-8 = output (interface solution z, and
+    // the next lane's first node xr), written by the solver warp before barrier 2 and read by every lane
+    // after it.  Inputs and outputs never share a plane, so one buffer is enough: the next solve's
+    // inputs are written after barrier 2 of this one, its outputs after its own barrier 1.
+    constexpr int G = 32 * W, PL_ = Comm<W>::SB_PLANE, ST_ = Comm<W>::SB_STRIDE;
+    const int g = cm.g;
+    double *sb = cm.sb;
+    const int me = Comm<W>::slot(g);
+    TRPL_DASSERT(me >= 0 && me < PL_ && g < G);
+    const double lr = l[M - 1];
+    sb[0 * PL_ + me] = y[0];
+    sb[1 * PL_ + me] = v[0];
+    sb[2 * PL_ + me] = w[0];
+    sb[3 * PL_ + me] = -lr * v[M - 2];                      // this lane's share of its interface row
+    sb[4 * PL_ + me] = fma(-lr, w[M - 2], d[M - 1]);
+    sb[5 * PL_ + me] = fma(-lr, y[M - 2], b[M - 1]);
+    sb[6 * PL_ + me] = u[M - 1];
+    __syncthreads();
+    if ((g >> 5) == cm.solver) {
+        const int sl_ = g & 31;                            // solver lane: rows W*sl_ .. W*sl_+W-1
+        double L2[W], D2[W], U2[W], B2[W], Z[W];
+#pragma unroll
+        for (int k = 0; k < W; k++) {
+            const int r = W * sl_ + k;                     // slot(r) = k * ST_ + sl_
+            const int here = k * ST_ + sl_;
+            const int next = (k + 1 < W) ? here + ST_ : ((sl_ < 31) ? sl_ + 1 : here);
+            const double ur = (r < G - 1) ? sb[6 * PL_ + here] : 0.0;
+            L2[k] = sb[3 * PL_ + here];
+            D2[k] = fma(-ur, sb[1 * PL_ + next], sb[4 * PL_ + here]);
+            U2[k] = -ur * sb[2 * PL_ + next];
+            B2[k] = fma(-ur, sb[0 * PL_ + next], sb[5 * PL_ + here]);
+        }
+        Comm<1> c1(sl_);
+        double znext;                                      // first row of the next lane
+        warp_solve<W, true>(L2, D2, U2, B2, Z, c1, znext);
+#pragma unroll
+        for (int k = 0; k < W; k++) {
+            const int here = k * ST_ + sl_;
+            const int next = (k + 1 < W) ? here + ST_ : ((sl_ < 31) ? sl_ + 1 : here);
+            const double zn = (k + 1 < W) ? Z[k + 1] : znext;
+            sb[7 * PL_ + here] = Z[k];
+            sb[8 * PL_ + here] = fma(-sb[2 * PL_ + next], zn, fma(-sb[1 * PL_ + next], Z[k], sb[0 * PL_ + next]));
+        }
+    }
+    __syncthreads();
+    cm.solver = (cm.solver + 1) & (W - 1);     // the role rotates: every scheduler gets its share of the serial part
+    const double z = sb[7 * PL_ + me];
+    const double zl = (g > 0) ? sb[7 * PL_ + Comm<W>::slot(g - 1)] : 0.0;
+    xr = (g < G - 1) ? sb[8 * PL_ + me] : 0.0;
+    x[M - 1] = z;
+#pragma unroll
+    for (int j = 0; j < M - 1; j++) x[j] = fma(-w[j], z, fma(-v[j], zl, y[j]));
+    return zl;
+}
+
+template <int M, int W>
+__device__ __forceinline__ double tridiag_solve(const double (&l)[M], const double (&d)[M],
+                                                const double (&u)[M], const double (&b)[M],
+                                                double (&x)[M], Comm<W> &cm, double &xr)
+{
+    if constexpr (W == 1) return warp_solve<M, false>(l, d, u, b, x, cm, xr);
+    else return cta_solve<M, W>(l, d, u, b, x, cm, xr);
 }
 
 // [sec:none]
@@ -417,7 +447,6 @@ __device__ __forceinline__ void run_sim(const KArgs &a, const int c, const long 
     const bool emu32 = (flags & TRPL_F_EMULATE_F32) != 0;
 
     // ---- parameters: non-dimensionalise (pvSimPCR.py:327-331), one column per lane, then broadcast
-#if TRPL_CONST_TABLE
     // Every per-simulation constant, raw or derived, is computed once, parked in one lane of `ctab`
     // and read back with a constant-lane shuffle: ptxas proves such a value warp-uniform and can
     // hold it in a uniform register; a derived constant it could recompute (tauP*N0P0 ...) would be
@@ -456,21 +485,6 @@ __device__ __forceinline__ void run_sim(const KArgs &a, const int c, const long 
     const double LamDP = __shfl_sync(FULL, ctab, 17), LamDN = __shfl_sync(FULL, ctab, 18);
     const double hLamDP = __shfl_sync(FULL, ctab, 19), hLamDN = __shfl_sync(FULL, ctab, 20);
     const double mLN0P0 = __shfl_sync(FULL, ctab, 21);   // pvSimPCR.py:278
-#else
-    double mpl = 0.0;
-    if (lane < TRPL_NPAR) mpl = a.x[s * a.ldx + lane] * cv.scales[lane];
-    const double N0 = __shfl_sync(FULL, mpl, 0), P0 = __shfl_sync(FULL, mpl, 1);
-    const double DN = __shfl_sync(FULL, mpl, 2), DP = __shfl_sync(FULL, mpl, 3);
-    const double rate = __shfl_sync(FULL, mpl, 4);
-    const double sr0 = __shfl_sync(FULL, mpl, 5), srL = __shfl_sync(FULL, mpl, 6);
-    const double CN = __shfl_sync(FULL, mpl, 7), CP = __shfl_sync(FULL, mpl, 8);
-    const double tauN = __shfl_sync(FULL, mpl, 9), tauP = __shfl_sync(FULL, mpl, 10);
-    const double Lam = __shfl_sync(FULL, mpl, 11);
-    const double N0P0 = N0 * P0;
-    const double hDN = 0.5 * DN, hDP = 0.5 * DP;
-    const double LamDP = Lam * DP, LamDN = Lam * DN, hLamDP = 0.5 * LamDP, hLamDN = 0.5 * LamDN;
-    const double mLN0P0 = -(double)L * N0P0;   // pvSimPCR.py:278
-#endif
     const double TOL = a.TOL;
     const double mag = (a.mag_col >= 0) ? a.x[s * a.ldx + a.mag_col] : 0.0;
 
@@ -542,11 +556,14 @@ __device__ __forceinline__ void run_sim(const KArgs &a, const int c, const long 
     double keep = 0.0;          // PL sample staged in this lane
     double lp_carry = 0.0;      // log PL of the sample preceding the current block of 32
     double pl0 = 1.0;           // PL(t=0) for self-normalisation
-    long long iters_total = 0;
-    int status = 0;
-    int pl_idx = 0;             // index of the next PL sample
-    int t_next_pl = 0;
 
+    // PL sample i of this simulation into the caller's buffer (f32 or f64)
+    auto store_pl = [&](const int i, const double v) {
+        if (a.pl_dtype == TRPL_F32)
+            reinterpret_cast<float *>(cv.pl_out)[s * a.pl_stride + i] = (float)v;
+        else
+            reinterpret_cast<double *>(cv.pl_out)[s * a.pl_stride + i] = v;
+    };
     // consume a block of `cnt` staged PL samples starting at index idx0
     // [sec:step-flush]
     auto flush = [&](const int idx0, const int cnt) {
@@ -558,12 +575,7 @@ __device__ __forceinline__ void run_sim(const KArgs &a, const int c, const long 
         } else {
             val = keep / cv.redim;
         }
-        if (cv.pl_out != nullptr && lane < cnt) {
-            if (a.pl_dtype == TRPL_F32)
-                reinterpret_cast<float *>(cv.pl_out)[s * a.pl_stride + idx0 + lane] = (float)val;
-            else
-                reinterpret_cast<double *>(cv.pl_out)[s * a.pl_stride + idx0 + lane] = val;
-        }
+        if (cv.pl_out != nullptr && lane < cnt) store_pl(idx0 + lane, val);
         if (a.E == 0) return;
         if (flags & TRPL_F_SELF_NORMALIZE) {
             if (idx0 == 0) pl0 = __shfl_sync(FULL, val, 0);
@@ -623,12 +635,126 @@ __device__ __forceinline__ void run_sim(const KArgs &a, const int c, const long 
         __syncwarp();
     };
 
+    // Newton system of one species with the other one frozen (pvSimPCR.py:147-216): l, d, u, b of X and
+    // the stop-rule partial sum z = sum(|residual| - TOL*|b|) of the current iterate (err < TOL <=> z < 0).
+    // `species` is std::true_type for the N system (X = N, Y = P) and std::false_type for the P system
+    // (X = P, Y = N); every product of N and P keeps its N-first operand order.
+    // -ds = X*(B + CP*P + CN*N) + C_X*np + srh: the factor B + CP*P + CN*N is shared with the rhs, and no
+    // product of two per-simulation constants appears inside the loop (see ctab above).  The SRH
+    // numerator (for N: P*tp - tauP*np) is evaluated as the equal tauN*P^2 + tauP*N0P0 (one product
+    // fewer, no cancellation).
+    // [sec:assembly]
+    auto assemble = [&](auto species, const double a0, const double (&bX)[M], const double Xl, const double Xr,
+                        const double En, double (&l)[M], double (&d)[M], double (&u)[M], double (&b)[M]) {
+        constexpr bool IS_N = decltype(species)::value;
+        const double (&X)[M] = IS_N ? N : P;
+        const double (&Y)[M] = IS_N ? P : N;
+        const double tX = IS_N ? tauP : tauN, tY = IS_N ? tauN : tauP;
+        const double tX_N0P0 = IS_N ? tauP_N0P0 : tauN_N0P0;
+        const double CX = IS_N ? CN : CP, CY = IS_N ? CP : CN;
+        double nds_[M];
+#pragma unroll
+        for (int j = 0; j < M; j++) {
+            const double Xj = X[j], Yj = Y[j];
+            const double yt = Yj * tY;
+            const double tp = fma(Xj, tX, yt);
+            const double npp = IS_N ? fma(Xj, Yj, -N0P0) : fma(Yj, Xj, -N0P0);
+            const double r = rcp64(tp);
+            const double qr = fma(yt, Yj, tX_N0P0) * r;
+            const double hr = fma(CY, Yj, CX * Xj) + rate;
+            const double nds = fma(Yj, hr, fma(CX, npp, qr * r));               // = -ds
+            nds_[j] = nds;
+            b[j] = fma(nds, Xj, -fma(hr + r, npp, bX[j]));
+        }
+        // transport rows.  The diagonal takes exactly the rounded off-diagonals of the two
+        // neighbouring rows (d_j = a0 - u_{j-1} - l_{j+1} - ds, pvSimPCR.py:159): the column sums of
+        // the transport part vanish in floating point, i.e. the step conserves carriers to the
+        // last bit -- a diagonal rebuilt from E differences does not, and that noise ends up in
+        // PL = rate*(sum N*P - L*N0*P0) once the excess has decayed (measured: stiff-regime agreement
+        // with the CPU restatement 96.9 % -> 94.9 %, profiles/r02_variants.txt).
+        {
+            const double D = IS_N ? DN : DP;
+            const double hDu = IS_N ? -hDN : hDP;    // D/2 with the sign of the field term in u
+            const double cu0 = sel(ev[0], fma(hDu, E[0], -D), 0.0);      // u of the previous lane's last row
+            const double clM = sel(ev[M], fma(-hDu, En, -D), 0.0);         // l of the next lane's first row
+#pragma unroll
+            for (int j = 0; j < M; j++) {
+                const double Ep = (j < M - 1) ? E[j + 1] : En;
+                l[j] = fma(-hDu, E[j], -D);                                      // N: DN*(+E/2 - 1), P: DP*(-E/2 - 1)
+                u[j] = fma(hDu, Ep, -D);                                        // N: DN*(-E/2 - 1), P: DP*(+E/2 - 1)
+                if (PAD) {
+                    l[j] = sel(nv[j] && ev[j], l[j], 0.0);
+                    u[j] = sel(nv[j] && ev[j + 1], u[j], 0.0);
+                }
+            }
+            if (!PAD) {
+                l[0] = sel(ev[0], l[0], 0.0);
+                u[M - 1] = sel(ev[M], u[M - 1], 0.0);
+            }
+#pragma unroll
+            for (int j = 0; j < M; j++)
+                d[j] = ((a0 - ((j == 0) ? cu0 : u[j - 1])) - ((j == M - 1) ? clM : l[j + 1])) + nds_[j];
+        }
+        // [sec:surface] surface recombination rows (pvSimPCR.py:164-170) + missing-neighbour fix
+        {
+            double Nb = N[M - 1], Pb = P[M - 1];        // back-surface node of this lane
+            if (PAD) {
+#pragma unroll
+                for (int j = 0; j < M - 1; j++) { Nb = (j == jl) ? N[j] : Nb; Pb = (j == jl) ? P[j] : Pb; }
+            }
+            const double Ns = is_first ? N[0] : Nb;
+            const double Ps = is_first ? P[0] : Pb;
+            const double Xs = IS_N ? Ns : Ps, Ys = IS_N ? Ps : Ns;
+            const double rs = rcp64(Ns + Ps);
+            const double srs = srf * rs;
+            const double nd = fma(Ys, Ys, N0P0) * (srs * rs);                   // = -ds0
+            const double db = fma(-nd, Xs, fma(Ns, Ps, -N0P0) * srs);
+            if (PAD) {
+#pragma unroll
+                for (int j = 0; j < M; j++) {
+                    const bool at = (is_first && j == 0) || (is_last && j == jl);
+                    d[j] += at ? nd : 0.0;
+                    b[j] -= at ? db : 0.0;
+                }
+            } else {
+                d[0] += is_first ? nd : 0.0;
+                b[0] -= is_first ? db : 0.0;
+                d[M - 1] += is_last ? nd : 0.0;
+                b[M - 1] -= is_last ? db : 0.0;
+            }
+        }
+        if (PAD) {
+#pragma unroll
+            for (int j = 0; j < M; j++) {
+                d[j] = sel(nv[j], d[j], 1.0);
+                b[j] = sel(nv[j], b[j], 0.0);
+            }
+        }
+        // [sec:residual] L1 residual of the current iterate         (pvSimPCR.py:172, :14-40)
+        double z = 0.0;
+#pragma unroll
+        for (int j = 0; j < M; j++) {
+            const double xm = (j == 0) ? Xl : X[j - 1];
+            const double xp = (j == M - 1) ? Xr : X[j + 1];
+            const double res = fma(l[j], xm, fma(d[j], X[j], fma(u[j], xp, -b[j])));
+            z = fma(-TOL, fabs(b[j]), z + fabs(res));
+        }
+        if (PADM == 1) z = dummy ? 0.0 : z;
+        return z;
+    };
+
     // =========================================================================================
     // time loop (pvSimPCR.py:237-293): t = 0 .. t_last, PL(t) emitted from the state at time t
     // =========================================================================================
     // [sec:step]
+    // time-loop state.  The declaration order matters to ptxas: other orders change the register
+    // assignment of the fine-grid kernel (+5 three-register DFMAs, profiles/r03_refactor_sass_budget.txt).
     bool failed = false;
+    int t_next_pl = 0;
     int t;
+    int pl_idx = 0;             // index of the next PL sample
+    int status = 0;
+    long long iters_total = 0;
     for (t = 0; t <= t_last; t++) {
         // [sec:step-PL] ---- PL(t) = rate * (sum_n N*P - L*N0*P0)             (pvSimPCR.py:276-281)
         bool emitted = false;
@@ -692,202 +818,21 @@ __device__ __forceinline__ void run_sim(const KArgs &a, const int c, const long 
         bool nonfinite = false;
         for (;;) {
             double l[M], d[M], u[M], b[M];
-            double zN = 0.0, zP = 0.0;    // sum(|residual| - TOL*|b|): err < TOL  <=>  z < 0
             bool converged_now = false, nonfinite_now = false;
-
-            // Assembly notes (both species).  -ds = X*(B + CP*P + CN*N) + C_X*np + srh (X = the other
-            // species): the factor B + CP*P + CN*N is shared with the rhs, and no product of two
-            // per-simulation constants appears inside the loop (see ctab above).  With the constant table
-            // the SRH numerator P*tp - tauP*np is evaluated as the equal tauN*P^2 + tauP*N0P0 (one product
-            // fewer, no cancellation).
-
-            // [sec:N-assembly] ======== N system (P, E frozen) ========
-            {
-                double nds_[M];
-#pragma unroll
-                for (int j = 0; j < M; j++) {
-                    const double Nj = N[j], Pj = P[j];
-                    const double pt = Pj * tauN;
-                    const double tp = fma(Nj, tauP, pt);
-                    const double npp = fma(Nj, Pj, -N0P0);
-                    const double r = rcp64(tp);
-#if TRPL_CONST_TABLE
-                    const double qr = fma(pt, Pj, tauP_N0P0) * r;
-#else
-                    const double qr = fma(-tauP, npp, Pj * tp) * r;
-#endif
-                    const double hr = fma(CP, Pj, CN * Nj) + rate;
-                    const double nds = fma(Pj, hr, fma(CN, npp, qr * r));               // = -ds
-                    nds_[j] = nds;
-                    b[j] = fma(nds, Nj, -fma(hr + r, npp, bN[j]));
-                }
-                // transport rows.  The diagonal takes exactly the rounded off-diagonals of the two
-                // neighbouring rows (d_j = a0 - u_{j-1} - l_{j+1} - ds, pvSimPCR.py:159): the column sums of
-                // the transport part vanish in floating point, i.e. the step conserves carriers to the
-                // last bit -- a diagonal rebuilt from E differences does not, and that noise ends up in
-                // PL = rate*(sum N*P - L*N0*P0) once the excess has decayed (measured: stiff-regime agreement
-                // with the CPU restatement 96.9 % -> 94.9 %, profiles/r02_variants.txt).
-                {
-                    const double cu0 = sel(ev[0], fma(-hDN, E[0], -DN), 0.0);      // u of the previous lane's last row
-                    const double clM = sel(ev[M], fma(hDN, En, -DN), 0.0);         // l of the next lane's first row
-#pragma unroll
-                    for (int j = 0; j < M; j++) {
-                        const double Ep = (j < M - 1) ? E[j + 1] : En;
-                        l[j] = fma(hDN, E[j], -DN);                                      // DN*(+E/2 - 1)
-                        u[j] = fma(-hDN, Ep, -DN);                                       // DN*(-E/2 - 1)
-                        if (PAD) {
-                            l[j] = sel(nv[j] && ev[j], l[j], 0.0);
-                            u[j] = sel(nv[j] && ev[j + 1], u[j], 0.0);
-                        }
-                    }
-                    if (!PAD) {
-                        l[0] = sel(ev[0], l[0], 0.0);
-                        u[M - 1] = sel(ev[M], u[M - 1], 0.0);
-                    }
-#pragma unroll
-                    for (int j = 0; j < M; j++)
-                        d[j] = ((a0 - ((j == 0) ? cu0 : u[j - 1])) - ((j == M - 1) ? clM : l[j + 1])) + nds_[j];
-                }
-                // [sec:N-surface] surface recombination rows (pvSimPCR.py:164-170) + missing-neighbour fix
-                {
-                    double Nb = N[M - 1], Pb = P[M - 1];        // back-surface node of this lane
-                    if (PAD) {
-#pragma unroll
-                        for (int j = 0; j < M - 1; j++) { Nb = (j == jl) ? N[j] : Nb; Pb = (j == jl) ? P[j] : Pb; }
-                    }
-                    const double Ns = is_first ? N[0] : Nb;
-                    const double Ps = is_first ? P[0] : Pb;
-                    const double rs = rcp64(Ns + Ps);
-                    const double srs = srf * rs;
-                    const double nd = fma(Ps, Ps, N0P0) * (srs * rs);                   // = -ds0
-                    const double db = fma(-nd, Ns, fma(Ns, Ps, -N0P0) * srs);
-                    if (PAD) {
-#pragma unroll
-                        for (int j = 0; j < M; j++) {
-                            const bool at = (is_first && j == 0) || (is_last && j == jl);
-                            d[j] += at ? nd : 0.0;
-                            b[j] -= at ? db : 0.0;
-                        }
-                    } else {
-                        d[0] += is_first ? nd : 0.0;
-                        b[0] -= is_first ? db : 0.0;
-                        d[M - 1] += is_last ? nd : 0.0;
-                        b[M - 1] -= is_last ? db : 0.0;
-                    }
-                }
-                if (PAD) {
-#pragma unroll
-                    for (int j = 0; j < M; j++) {
-                        d[j] = sel(nv[j], d[j], 1.0);
-                        b[j] = sel(nv[j], b[j], 0.0);
-                    }
-                }
-                // [sec:N-residual] L1 residual of the current iterate         (pvSimPCR.py:172, :14-40)
-#pragma unroll
-                for (int j = 0; j < M; j++) {
-                    const double xm = (j == 0) ? Nl : N[j - 1];
-                    const double xp = (j == M - 1) ? Nr : N[j + 1];
-                    const double res = fma(l[j], xm, fma(d[j], N[j], fma(u[j], xp, -b[j])));
-                    zN = fma(-TOL, fabs(b[j]), zN + fabs(res));
-                }
-                if (PADM == 1) zN = dummy ? 0.0 : zN;
-                // [sec:N-solve]
-                Nl = tridiag_solve<M, W>(l, d, u, b, N, cm, Nr);
-            }
-
-            // [sec:P-assembly] ======== P system (new N) ========
-            {
-                double nds_[M];
-#pragma unroll
-                for (int j = 0; j < M; j++) {
-                    const double Nj = N[j], Pj = P[j];
-                    const double nt = Nj * tauP;
-                    const double tp = fma(Pj, tauN, nt);
-                    const double npp = fma(Nj, Pj, -N0P0);
-                    const double r = rcp64(tp);
-#if TRPL_CONST_TABLE
-                    const double qr = fma(nt, Nj, tauN_N0P0) * r;
-#else
-                    const double qr = fma(-tauN, npp, Nj * tp) * r;
-#endif
-                    const double hr = fma(CN, Nj, CP * Pj) + rate;
-                    const double nds = fma(Nj, hr, fma(CP, npp, qr * r));
-                    nds_[j] = nds;
-                    b[j] = fma(nds, Pj, -fma(hr + r, npp, bP[j]));
-                }
-                {
-                    const double cu0 = sel(ev[0], fma(hDP, E[0], -DP), 0.0);
-                    const double clM = sel(ev[M], fma(-hDP, En, -DP), 0.0);
-#pragma unroll
-                    for (int j = 0; j < M; j++) {
-                        const double Ep = (j < M - 1) ? E[j + 1] : En;
-                        l[j] = fma(-hDP, E[j], -DP);                                     // DP*(-E/2 - 1)
-                        u[j] = fma(hDP, Ep, -DP);                                        // DP*(+E/2 - 1)
-                        if (PAD) {
-                            l[j] = sel(nv[j] && ev[j], l[j], 0.0);
-                            u[j] = sel(nv[j] && ev[j + 1], u[j], 0.0);
-                        }
-                    }
-                    if (!PAD) {
-                        l[0] = sel(ev[0], l[0], 0.0);
-                        u[M - 1] = sel(ev[M], u[M - 1], 0.0);
-                    }
-#pragma unroll
-                    for (int j = 0; j < M; j++)
-                        d[j] = ((a0 - ((j == 0) ? cu0 : u[j - 1])) - ((j == M - 1) ? clM : l[j + 1])) + nds_[j];
-                }
-                // [sec:P-surface]
-                {
-                    double Nb = N[M - 1], Pb = P[M - 1];
-                    if (PAD) {
-#pragma unroll
-                        for (int j = 0; j < M - 1; j++) { Nb = (j == jl) ? N[j] : Nb; Pb = (j == jl) ? P[j] : Pb; }
-                    }
-                    const double Ns = is_first ? N[0] : Nb;
-                    const double Ps = is_first ? P[0] : Pb;
-                    const double rs = rcp64(Ns + Ps);
-                    const double srs = srf * rs;
-                    const double nd = fma(Ns, Ns, N0P0) * (srs * rs);
-                    const double db = fma(-nd, Ps, fma(Ns, Ps, -N0P0) * srs);
-                    if (PAD) {
-#pragma unroll
-                        for (int j = 0; j < M; j++) {
-                            const bool at = (is_first && j == 0) || (is_last && j == jl);
-                            d[j] += at ? nd : 0.0;
-                            b[j] -= at ? db : 0.0;
-                        }
-                    } else {
-                        d[0] += is_first ? nd : 0.0;
-                        b[0] -= is_first ? db : 0.0;
-                        d[M - 1] += is_last ? nd : 0.0;
-                        b[M - 1] -= is_last ? db : 0.0;
-                    }
-                }
-                if (PAD) {
-#pragma unroll
-                    for (int j = 0; j < M; j++) {
-                        d[j] = sel(nv[j], d[j], 1.0);
-                        b[j] = sel(nv[j], b[j], 0.0);
-                    }
-                }
-                // [sec:P-residual]
-#pragma unroll
-                for (int j = 0; j < M; j++) {
-                    const double xm = (j == 0) ? Pl : P[j - 1];
-                    const double xp = (j == M - 1) ? Pr : P[j + 1];
-                    const double res = fma(l[j], xm, fma(d[j], P[j], fma(u[j], xp, -b[j])));
-                    zP = fma(-TOL, fabs(b[j]), zP + fabs(res));
-                }
-                // [sec:stop-rule] ---- stop decision for THIS iteration (pvSimPCR.py:213-216): both L1
-                // residuals are known here, before the P solve; reducing them now lets the shuffle
-                // chain overlap the solve.
-                if (PADM == 1) zP = dummy ? 0.0 : zP;
-                if constexpr (W == 1) cm.stop_rule(zN, zP, converged_now, nonfinite_now);
-                else cm.stop_post(zN, zP);
-                // [sec:P-solve]
-                Pl = tridiag_solve<M, W>(l, d, u, b, P, cm, Pr);
-                if constexpr (W > 1) cm.stop_collect(converged_now, nonfinite_now);
-            }
+            // [sec:N] ======== N system (P, E frozen) ========
+            const double zN = assemble(std::true_type(), a0, bN, Nl, Nr, En, l, d, u, b);
+            // [sec:N-solve]
+            Nl = tridiag_solve<M, W>(l, d, u, b, N, cm, Nr);
+            // [sec:P] ======== P system (new N) ========
+            const double zP = assemble(std::false_type(), a0, bP, Pl, Pr, En, l, d, u, b);
+            // [sec:stop-rule] ---- stop decision for THIS iteration (pvSimPCR.py:213-216): both L1
+            // residuals are known here, before the P solve; reducing them now lets the shuffle
+            // chain overlap the solve.
+            if constexpr (W == 1) cm.stop_rule(zN, zP, converged_now, nonfinite_now);
+            else cm.stop_post(zN, zP);
+            // [sec:P-solve]
+            Pl = tridiag_solve<M, W>(l, d, u, b, P, cm, Pr);
+            if constexpr (W > 1) cm.stop_collect(converged_now, nonfinite_now);
 
             // [sec:E-update] ======== E update on interior edges             (pvSimPCR.py:205-209)
 #pragma unroll
@@ -930,12 +875,7 @@ __device__ __forceinline__ void run_sim(const KArgs &a, const int c, const long 
     if (io_warp && (pl_idx & 31)) flush(pl_idx & ~31, pl_idx & 31);
     if (io_warp && failed && cv.pl_out != nullptr) {
         const double qnan = __longlong_as_double(0x7ff8000000000000LL);
-        for (int i = pl_idx + lane; i < n_pl; i += 32) {
-            if (a.pl_dtype == TRPL_F32)
-                reinterpret_cast<float *>(cv.pl_out)[s * a.pl_stride + i] = (float)qnan;
-            else
-                reinterpret_cast<double *>(cv.pl_out)[s * a.pl_stride + i] = qnan;
-        }
+        for (int i = pl_idx + lane; i < n_pl; i += 32) store_pl(i, qnan);
     }
 
     // ---- results
@@ -955,7 +895,7 @@ __device__ __forceinline__ void run_sim(const KArgs &a, const int c, const long 
 
 // [sec:kernel]
 template <int M, bool PAD>
-__global__ void __launch_bounds__(WARPS_PER_CTA * 32, TRPL_MIN_CTAS)
+__global__ void __launch_bounds__(WARPS_PER_CTA * 32, MIN_CTAS_PER_SM)
 trpl_sim_kernel(const __grid_constant__ KArgs a)
 {
     extern __shared__ __align__(16) double smem[];
@@ -964,8 +904,7 @@ trpl_sim_kernel(const __grid_constant__ KArgs a)
     double *ring_warp = smem + (size_t)warp * (4 * 3 * M * 32 + RING_CANARY);
     if (TRPL_DEBUG && lane == 0) reinterpret_cast<unsigned long long *>(ring_warp + 4 * 3 * M * 32)[0] = CANARY_WORD;
     const unsigned long long total = (unsigned long long)a.S * (unsigned long long)a.C;
-    Comm<1> cm;
-    cm.g = lane; cm.xb = nullptr; cm.red = nullptr; cm.phase = 0; cm.rphase = 0; cm.sb = nullptr; cm.solver = 0;
+    Comm<1> cm(lane);
     for (;;) {
         unsigned long long item = 0;
         if (lane == 0) item = atomicAdd(a.counter, 1ULL);
@@ -991,12 +930,7 @@ trpl_sim_cta_kernel(const __grid_constant__ KArgs a)
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     double *ring_warp = smem + (size_t)warp * (4 * 3 * M * 32 + RING_CANARY);
     if (TRPL_DEBUG && lane == 0) reinterpret_cast<unsigned long long *>(ring_warp + 4 * 3 * M * 32)[0] = CANARY_WORD;
-    Comm<W> cm;
-    cm.g = threadIdx.x;
-    cm.xb = smem + (size_t)W * (4 * 3 * M * 32 + RING_CANARY);
-    cm.red = cm.xb + 2 * Comm<W>::XB_K * 32 * W;
-    cm.sb = cm.red + 2 * W * 4;
-    cm.phase = 0; cm.rphase = 0; cm.solver = blockIdx.x & (W - 1);
+    Comm<W> cm(threadIdx.x, smem + (size_t)W * (4 * 3 * M * 32 + RING_CANARY), blockIdx.x & (W - 1));
     const unsigned long long total = (unsigned long long)a.S * (unsigned long long)a.C;
     for (;;) {
         __syncthreads();

@@ -5,10 +5,16 @@ library with inline line info:
     cuobjdump -xelf all bayesian_inference_trpl_b200/libtrpl_b200.so
     nvdisasm -gi -c trpl_kernels.sm_100a.cubin > lined.sass
     python profiles/sass_budget.py lined.sass trpl_sim_kernelILi4ELb0 [--dump newton.sass]
+    LOOP_MIN=300 LOOP_MAX=8000 python profiles/sass_budget.py lined.sass trpl_sim_cta_kernelILi4ELi8ELi1
+
+The Newton loop is the FP64-densest loop of LOOP_MIN..LOOP_MAX instructions (default 400..1600, which
+fits the warp kernel at M <= 4); LOOP_MIN=300 LOOP_MAX=8000 covers every trpl_sim_kernel and
+trpl_sim_cta_kernel instantiation.
 
 Every instruction of the innermost big loop (the Newton / Gauss-Seidel iteration) is attributed to
-a section of `run_sim` / `tridiag_solve` through the source lines marked `// [sec:NAME]` in
-csrc/trpl_solver.cuh, and counted by kind:
+a section of csrc/trpl_solver.cuh through the source lines marked `// [sec:NAME]` there, and counted
+by kind.  Code inlined from a helper (the species assembly, the tridiagonal solve) is named by its
+call site plus the helper's own section, e.g. `N:surface` or `P-solve:pcr`.  Kinds:
   DFMA / DMUL / DADD      FP64 pipe, 2 issue cycles per warp instruction on an SMSP
   3reg                    DFMAs whose three sources are distinct vector registers without a .reuse
                           hit: 3 cycles (register-bank limit, profiles/r01_microbench.txt)
@@ -104,16 +110,14 @@ if outer:
 
 
 def section(chain):
-    # outermost frame inside the solver file decides; tridiag_solve frames refine it
+    # the outermost tagged frame (the call site in run_sim) names the row; the innermost one refines it
     secs = [sec_of_line.get(line) for f, line in chain if f.endswith(SOLVER)]
     secs = [s for s in secs if s and s not in ("kernel", "none")]
     if not secs:
         return "other"
     outer = secs[-1]
     inner = secs[0]
-    if outer in ("N-solve", "P-solve") and inner != outer:
-        return outer + ":" + inner
-    return outer
+    return outer if inner == outer else outer + ":" + inner
 
 
 ALU = {"FSEL", "LOP3", "ISETP", "VIMNMX", "SEL", "IADD3", "VIADD", "PLOP3", "SHF", "LEA", "ISCADD", "IABS",

@@ -1,7 +1,9 @@
 #!/usr/bin/env python3
-"""Build A/B variants of libtrpl_b200.so into build/variants/ (shipped to the GPU box, git-ignored):
-    python tools/build_variants.py name:-DFLAG=1,-DOTHER=2 ...  [head]
-`head` builds the kernel sources of git HEAD (the previous round's shipped kernel) as the baseline."""
+"""Build variants of libtrpl_b200.so into build/variants/ (git-ignored) for A/B runs:
+    python tools/build_variants.py name[:-DFLAG=1,...] ...  [head[@rev]]
+`name` builds the working tree with the given extra nvcc flags; the only flag that selects other
+code is -DTRPL_DEBUG=1 (device-side checks, e.g. `debug:-DTRPL_DEBUG=1`).  `head` builds the kernel
+sources of git HEAD (or of `rev`) as the baseline."""
 import os
 import subprocess
 import sys
