@@ -13,11 +13,10 @@ LIB_PATH = os.environ.get("TRPL_LIB", os.path.join(_PKG, "libtrpl_b200.so"))   #
 SRC = os.path.join(_PKG, "csrc", "trpl_kernels.cu")
 INCLUDE = os.path.join(_ROOT, "include")
 
-NPAR = 12
 MAX_CURVES = 8
 MAX_EXP = 4
+OK, EINVAL, EUNSUPPORTED, ECUDA, ENODEVICE = 0, -1, -2, -3, -4
 F64, F32 = 0, 1
-ST_NOCONV, ST_NONFINITE = 1, 2
 F_INIT_GRID_UNITS, F_LOG_PL, F_SELF_NORMALIZE, F_EMULATE_F32 = 1, 2, 4, 8
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
@@ -37,6 +36,33 @@ class Obs(ctypes.Structure):
 class Curve(ctypes.Structure):
     _fields_ = [("d_init", ctypes.c_void_p), ("length", ctypes.c_double),
                 ("obs", Obs * MAX_EXP)]
+
+
+_vp, _int, _i64, _u64, _dbl = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_uint64, ctypes.c_double
+
+# name -> (restype, argtypes) of every export, in the order of include/trpl_b200.h
+_SIGNATURES = {
+    "trpl_version": (_int, []),
+    "trpl_error_string": (ctypes.c_char_p, [_int]),
+    "trpl_last_cuda_error": (ctypes.c_char_p, []),
+    "trpl_resident_sims": (_int, [_int, _int]),
+    "trpl_solve_pl": (_int, [_vp, _i64, _i64, _vp, _dbl, _dbl, _int, _int, _int, _int, _int, _int, _int,
+                             _vp, _int, _i64, _vp, _vp, _int, _vp]),
+    "trpl_solve_loglik": (_int, [_vp, _i64, _i64, _int, ctypes.POINTER(Curve), _int, _int, _dbl, _int,
+                                 _int, _int, _int, _int, _int, _vp, _vp, _vp, _vp, _int, _vp]),
+    "trpl_log10_clamp": (_int, [_vp, _int, _i64, _dbl, _int, _vp]),
+    "trpl_lnp_accumulate": (_int, [_vp, _vp, _i64, _i64, _i64, _vp, _vp, _int, _vp]),
+    "trpl_obs_prepare": (_int, [_vp, _int, _dbl, _int, _vp, _vp, _vp]),
+    "trpl_lse_partial": (_int, [_vp, _i64, _vp, _int, _vp]),
+    "trpl_random_grid": (_int, [_vp, _i64, _i64, _vp, _vp, _vp, _int, _int, _u64, _u64, _int, _vp]),
+    "trpl_posterior_weights": (_int, [_vp, _i64, _dbl, _vp, _int, _vp]),
+    "trpl_weighted_hist": (_int, [_vp, _i64, _i64, _int, _int, _vp, _dbl, _dbl, _int, _dbl, _dbl, _int, _vp,
+                                  _int, _vp]),
+    "trpl_weighted_moments": (_int, [_vp, _i64, _i64, _int, _vp, _vp, _int, _vp]),
+    "trpl_selftest_rcp": (_int, [_vp, _vp, _i64, _int, _vp]),
+    "trpl_bench_dfma": (_int, [_int, _int, ctypes.POINTER(_dbl), ctypes.POINTER(_dbl)]),
+}
+EXPORTS = list(_SIGNATURES)
 
 
 def build(force=False, verbose=False):
@@ -72,55 +98,18 @@ def lib():
         raise TrplError("libtrpl_b200.so is not built: run `python -c 'import __graft_entry__ as g; "
                         "g.build()'` (needs nvcc). There is no CPU fallback.")
     L = ctypes.CDLL(LIB_PATH)
-    vp, i32, i64, dbl = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_double
-    L.trpl_version.restype = i32
-    L.trpl_error_string.restype = ctypes.c_char_p
-    L.trpl_error_string.argtypes = [i32]
-    L.trpl_last_cuda_error.restype = ctypes.c_char_p
-    L.trpl_resident_sims.restype = i32
-    L.trpl_resident_sims.argtypes = [i32, i32]
-    L.trpl_solve_pl.restype = i32
-    L.trpl_solve_pl.argtypes = [vp, i64, i64, vp, dbl, dbl, i32, i32, i32, i32, i32, i32, i32,
-                                vp, i32, i64, vp, vp, i32, vp]
-    L.trpl_solve_loglik.restype = i32
-    L.trpl_solve_loglik.argtypes = [vp, i64, i64, i32, ctypes.POINTER(Curve), i32, i32, dbl, i32,
-                                    i32, i32, i32, i32, i32, vp, vp, vp, vp, i32, vp]
-    L.trpl_log10_clamp.restype = i32
-    L.trpl_log10_clamp.argtypes = [vp, i32, i64, dbl, i32, vp]
-    L.trpl_lnp_accumulate.restype = i32
-    L.trpl_lnp_accumulate.argtypes = [vp, vp, i64, i64, i64, vp, vp, i32, vp]
-    L.trpl_obs_prepare.restype = i32
-    L.trpl_obs_prepare.argtypes = [vp, ctypes.c_int32, dbl, i32, vp, vp, vp]
-    L.trpl_lse_partial.restype = i32
-    L.trpl_lse_partial.argtypes = [vp, i64, vp, i32, vp]
-    u64 = ctypes.c_uint64
-    L.trpl_random_grid.restype = i32
-    L.trpl_random_grid.argtypes = [vp, i64, i64, vp, vp, vp, i32, i32, u64, u64, i32, vp]
-    L.trpl_posterior_weights.restype = i32
-    L.trpl_posterior_weights.argtypes = [vp, i64, dbl, vp, i32, vp]
-    L.trpl_weighted_hist.restype = i32
-    L.trpl_weighted_hist.argtypes = [vp, i64, i64, i32, i32, vp, dbl, dbl, i32, dbl, dbl, i32, vp, i32, vp]
-    L.trpl_weighted_moments.restype = i32
-    L.trpl_weighted_moments.argtypes = [vp, i64, i64, i32, vp, vp, i32, vp]
-    L.trpl_selftest_rcp.restype = i32
-    L.trpl_selftest_rcp.argtypes = [vp, vp, i64, i32, vp]
-    L.trpl_bench_dfma.restype = i32
-    L.trpl_bench_dfma.argtypes = [i32, i32, ctypes.POINTER(dbl), ctypes.POINTER(dbl)]
+    for name, (restype, argtypes) in _SIGNATURES.items():
+        fn = getattr(L, name)
+        fn.restype, fn.argtypes = restype, argtypes
     _lib = L
     return L
-
-
-EXPORTS = ["trpl_version", "trpl_error_string", "trpl_last_cuda_error", "trpl_resident_sims",
-           "trpl_solve_pl", "trpl_solve_loglik", "trpl_log10_clamp", "trpl_lnp_accumulate",
-           "trpl_obs_prepare", "trpl_lse_partial", "trpl_bench_dfma", "trpl_random_grid",
-           "trpl_posterior_weights", "trpl_weighted_hist", "trpl_weighted_moments", "trpl_selftest_rcp"]
 
 
 def check(rc, what):
     if rc < 0:
         L = lib()
         msg = L.trpl_error_string(rc).decode()
-        if rc == -3:
+        if rc == ECUDA:
             msg += " [" + L.trpl_last_cuda_error().decode() + "]"
         raise TrplError("%s failed: %s (code %d)" % (what, msg, rc))
     return rc

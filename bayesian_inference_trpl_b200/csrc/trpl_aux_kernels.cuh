@@ -25,37 +25,25 @@ __global__ void trpl_finish_kernel(const double *sse, double *lnl, const int *st
 }
 
 // ---- probs.fastlog / log_kernel (probs.py:64-85) ---------------------------------------------
-// HBM-bound streaming kernels: 4 independent loads in flight per thread (memory-level parallelism).
-__global__ void trpl_log10_kernel_f64(double *x, long long n, double mn)
+// Clamp and log of one element.  float32 follows the reference's float32 buffer: compare in double, clamp
+// to (float)min, log10f.
+__device__ __forceinline__ double clamp_min(double v, double mn) { return v < mn ? mn : v; }
+__device__ __forceinline__ float clamp_min(float v, double mn) { return (double)v < mn ? (float)mn : v; }
+__device__ __forceinline__ double log10_of(double v) { return log10(v); }
+__device__ __forceinline__ float log10_of(float v) { return log10f(v); }
+// HBM-bound streaming kernel: 4 independent loads in flight per thread (memory-level parallelism).  All four
+// are clamped before the first log: clamping each just before its log costs the float64 kernel 3 registers.
+template <class T>
+__global__ void trpl_log10_kernel(T *x, long long n, double mn)
 {
     const long long stride = (long long)gridDim.x * blockDim.x;
     long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     for (; i + 3 * stride < n; i += 4 * stride) {
-        double v0 = x[i], v1 = x[i + stride], v2 = x[i + 2 * stride], v3 = x[i + 3 * stride];
-        v0 = v0 < mn ? mn : v0; v1 = v1 < mn ? mn : v1; v2 = v2 < mn ? mn : v2; v3 = v3 < mn ? mn : v3;
-        x[i] = log10(v0); x[i + stride] = log10(v1); x[i + 2 * stride] = log10(v2); x[i + 3 * stride] = log10(v3);
+        const T v0 = clamp_min(x[i], mn), v1 = clamp_min(x[i + stride], mn);
+        const T v2 = clamp_min(x[i + 2 * stride], mn), v3 = clamp_min(x[i + 3 * stride], mn);
+        x[i] = log10_of(v0); x[i + stride] = log10_of(v1); x[i + 2 * stride] = log10_of(v2); x[i + 3 * stride] = log10_of(v3);
     }
-    for (; i < n; i += stride) {
-        double v = x[i];
-        if (v < mn) v = mn;
-        x[i] = log10(v);
-    }
-}
-__device__ __forceinline__ float log10_clamp_f32(float v, double mn)
-{
-    if ((double)v < mn) v = (float)mn;
-    return log10f(v);
-}
-__global__ void trpl_log10_kernel_f32(float *x, long long n, double mn)
-{
-    const long long stride = (long long)gridDim.x * blockDim.x;
-    long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    for (; i + 3 * stride < n; i += 4 * stride) {
-        const float v0 = x[i], v1 = x[i + stride], v2 = x[i + 2 * stride], v3 = x[i + 3 * stride];
-        x[i] = log10_clamp_f32(v0, mn); x[i + stride] = log10_clamp_f32(v1, mn);
-        x[i + 2 * stride] = log10_clamp_f32(v2, mn); x[i + 3 * stride] = log10_clamp_f32(v3, mn);
-    }
-    for (; i < n; i += stride) x[i] = log10_clamp_f32(x[i], mn);
+    for (; i < n; i += stride) x[i] = log10_of(clamp_min(x[i], mn));
 }
 
 // ---- probs.prob / kernel_lnP (probs.py:20-62): one warp per sample, coalesced row reads -------
@@ -86,38 +74,45 @@ __global__ void trpl_lnp_kernel(double *P, const double *pl, long long S, long l
 }
 
 // ---- shard-local log-sum-exp pieces (Visualization/utils.py:157-166) --------------------------
-__global__ void trpl_lse_max_kernel(const double *x, long long n, double *out)
+// Block reduction of one value per thread: xor butterfly 16 -> 1 in every warp, the warp partials through
+// shared memory, then a butterfly over them in warp 0.  Thread 0 holds the block's result.
+template <class Op>
+__device__ __forceinline__ double block_reduce(double v, double identity, Op op)
 {
     __shared__ double sh[32];
+#pragma unroll
+    for (int o = 16; o >= 1; o >>= 1) v = op(v, __shfl_xor_sync(FULL, v, o));
+    if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = v;
+    __syncthreads();
+    if (threadIdx.x < 32) {
+        v = (threadIdx.x < (blockDim.x >> 5)) ? sh[threadIdx.x] : identity;
+#pragma unroll
+        for (int o = 16; o >= 1; o >>= 1) v = op(v, __shfl_xor_sync(FULL, v, o));
+    }
+    return v;
+}
+__global__ void trpl_lse_max_kernel(const double *x, long long n, double *out)
+{
     double m = -INFINITY;
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += stride) {
         const double v = x[i];
         if (v == v && v > m) m = v;
     }
-#pragma unroll
-    for (int o = 16; o >= 1; o >>= 1) m = fmax(m, __shfl_xor_sync(FULL, m, o));
-    if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = m;
-    __syncthreads();
-    if (threadIdx.x < 32) {
-        m = (threadIdx.x < (blockDim.x >> 5)) ? sh[threadIdx.x] : -INFINITY;
-#pragma unroll
-        for (int o = 16; o >= 1; o >>= 1) m = fmax(m, __shfl_xor_sync(FULL, m, o));
-        if (threadIdx.x == 0) {
-            // atomic max on doubles via ordered-integer trick
-            unsigned long long *addr = reinterpret_cast<unsigned long long *>(out);
-            unsigned long long old = *addr, assumed;
-            do {
-                assumed = old;
-                if (__longlong_as_double((long long)assumed) >= m) break;
-                old = atomicCAS(addr, assumed, (unsigned long long)__double_as_longlong(m));
-            } while (assumed != old);
-        }
+    m = block_reduce(m, -INFINITY, [](double a, double b) { return fmax(a, b); });
+    if (threadIdx.x == 0) {
+        // atomic max on doubles via ordered-integer trick
+        unsigned long long *addr = reinterpret_cast<unsigned long long *>(out);
+        unsigned long long old = *addr, assumed;
+        do {
+            assumed = old;
+            if (__longlong_as_double((long long)assumed) >= m) break;
+            old = atomicCAS(addr, assumed, (unsigned long long)__double_as_longlong(m));
+        } while (assumed != old);
     }
 }
 __global__ void trpl_lse_sum_kernel(const double *x, long long n, double *out)
 {
-    __shared__ double sh[32];
     const double mx = out[0];
     double acc = 0.0;
     const long long stride = (long long)gridDim.x * blockDim.x;
@@ -125,14 +120,8 @@ __global__ void trpl_lse_sum_kernel(const double *x, long long n, double *out)
         const double v = x[i];
         if (v == v && v > -INFINITY) acc += exp(v - mx);   // -inf entries weigh 0 (also when every entry is -inf)
     }
-    acc = warp_sum(acc);
-    if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = acc;
-    __syncthreads();
-    if (threadIdx.x < 32) {
-        acc = (threadIdx.x < (blockDim.x >> 5)) ? sh[threadIdx.x] : 0.0;
-        acc = warp_sum(acc);
-        if (threadIdx.x == 0) atomicAdd(out + 1, acc);
-    }
+    acc = block_reduce(acc, 0.0, [](double a, double b) { return a + b; });
+    if (threadIdx.x == 0) atomicAdd(out + 1, acc);
 }
 __global__ void trpl_lse_init_kernel(double *out)
 {

@@ -56,6 +56,11 @@ int cuda_fail(cudaError_t e, const char *what)
         cudaError_t e_ = (call);                                   \
         if (e_ != cudaSuccess) return cuda_fail(e_, #call);        \
     } while (0)
+// propagates a TRPL_E* code of a host helper
+#define TRY(call)                                                  \
+    do {                                                           \
+        if (int rc_ = (call)) return rc_;                          \
+    } while (0)
 
 // pvSimPCR.py:327-331 (same expression order; pow() is glibc's, as in CPython)
 void make_scales(double length, double time, int L, int T, double *sc, double *dx_o, double *dt_o)
@@ -79,6 +84,28 @@ struct Scratch {
     Scratch(const Scratch &) = delete;
     Scratch &operator=(const Scratch &) = delete;
 };
+
+// CUDA event, destroyed on every exit path
+struct Event {
+    cudaEvent_t e = nullptr;
+    cudaError_t create() { return cudaEventCreate(&e); }
+    ~Event() { if (e) cudaEventDestroy(e); }
+    Event() = default;
+    Event(const Event &) = delete;
+    Event &operator=(const Event &) = delete;
+};
+
+// Grid of a grid-stride kernel over `work` items with `tb` threads per block: one item per thread, at most
+// `per_sm` blocks per SM of `device`.  The reductions accumulate one partial sum per block, so their grouping
+// (and last bits) follow this grid.
+int stride_grid(int device, long long work, int tb, int per_sm, unsigned *grid)
+{
+    int nsm = 0;
+    CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
+    const long long want = (work + tb - 1) / tb, cap = (long long)nsm * per_sm;
+    *grid = (unsigned)(want < cap ? want : cap);
+    return TRPL_OK;
+}
 
 struct Cfg { int M; bool pad; int W; };      // W = warps per simulation (1: warp kernel, >1: CTA kernel)
 int pick_cfg(int L, Cfg *cfg)
@@ -202,6 +229,16 @@ struct DeviceGuard {
     ~DeviceGuard() { if (switched) cudaSetDevice(prev); }
 };
 
+// Runs `work` (returning a TRPL_* code) with `device` current, or returns why the device cannot be entered.
+// Entry points validate their arguments before this and call it once, so every one has the same shape.
+template <class F>
+int on_device(int device, F &&work)
+{
+    DeviceGuard guard;
+    TRY(guard.enter(device));
+    return work();
+}
+
 int launch_sims(KArgs &ka, const Cfg &cfg, int device, cudaStream_t st)
 {
     Geometry geo;
@@ -254,15 +291,12 @@ const char *trpl_last_cuda_error(void) { return g_cuda_err; }
 int trpl_resident_sims(int device, int L)
 {
     Cfg cfg;
-    int rc = pick_cfg(L, &cfg);
-    if (rc) return rc;
-    DeviceGuard guard;
-    rc = guard.enter(device);
-    if (rc) return rc;
-    Geometry geo;
-    rc = kernel_geometry(device, cfg, &geo);
-    if (rc) return rc;
-    return geo.ctas_per_sm * geo.sms * geo.sims_per_cta;
+    TRY(pick_cfg(L, &cfg));
+    return on_device(device, [&] {
+        Geometry geo;
+        TRY(kernel_geometry(device, cfg, &geo));
+        return geo.ctas_per_sm * geo.sms * geo.sims_per_cta;
+    });
 }
 
 int trpl_solve_pl(const double *d_matpar, int64_t S, int64_t ld_matpar, const double *d_init,
@@ -275,26 +309,22 @@ int trpl_solve_pl(const double *d_matpar, int64_t S, int64_t ld_matpar, const do
         (pl_dtype != TRPL_F64 && pl_dtype != TRPL_F32))
         return TRPL_EINVAL;
     Cfg cfg;
-    int rc = pick_cfg(L, &cfg);
-    if (rc) return rc;
-    DeviceGuard guard;
-    rc = guard.enter(device);
-    if (rc) return rc;
-    if (S == 0) return TRPL_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-
-    KArgs ka;
-    init_kargs(ka, L, tol, max_iter, max_order);
-    ka.x = d_matpar; ka.ldx = ld_matpar; ka.S = S; ka.pl_stride = pl_stride;
-    ka.sse = nullptr; ka.status = d_status; ka.iters = (long long *)d_iters;
-    ka.mag_col = -1; ka.C = 1; ka.E = 0; ka.plT = plT;
-    ka.flags = (flags & TRPL_F_INIT_GRID_UNITS) | (pl_dtype == TRPL_F32 ? TRPL_F_EMULATE_F32 : 0);
-    ka.pl_dtype = pl_dtype;
-    CurveDev &cv = ka.curves[0];
-    init_curve(cv, length, time, L, T, flags, d_init);
-    cv.pl_out = d_pl;
-    cv.t_last = T;
-    return launch_sims(ka, cfg, device, st);
+    TRY(pick_cfg(L, &cfg));
+    return on_device(device, [&] {
+        if (S == 0) return TRPL_OK;
+        KArgs ka;
+        init_kargs(ka, L, tol, max_iter, max_order);
+        ka.x = d_matpar; ka.ldx = ld_matpar; ka.S = S; ka.pl_stride = pl_stride;
+        ka.sse = nullptr; ka.status = d_status; ka.iters = (long long *)d_iters;
+        ka.mag_col = -1; ka.C = 1; ka.E = 0; ka.plT = plT;
+        ka.flags = (flags & TRPL_F_INIT_GRID_UNITS) | (pl_dtype == TRPL_F32 ? TRPL_F_EMULATE_F32 : 0);
+        ka.pl_dtype = pl_dtype;
+        CurveDev &cv = ka.curves[0];
+        init_curve(cv, length, time, L, T, flags, d_init);
+        cv.pl_out = d_pl;
+        cv.t_last = T;
+        return launch_sims(ka, cfg, device, (cudaStream_t)stream);
+    });
 }
 
 int trpl_solve_loglik(const double *d_x, int64_t S, int64_t ldx, int mag_col,
@@ -307,87 +337,75 @@ int trpl_solve_loglik(const double *d_x, int64_t S, int64_t ldx, int mag_col,
         return TRPL_EINVAL;
     if (C > TRPL_MAX_CURVES || E > TRPL_MAX_EXP) return TRPL_EUNSUPPORTED;
     Cfg cfg;
-    int rc = pick_cfg(L, &cfg);
-    if (rc) return rc;
-    DeviceGuard guard;
-    rc = guard.enter(device);
-    if (rc) return rc;
-    if (S == 0) return TRPL_OK;
-    cudaStream_t st = (cudaStream_t)stream;
+    TRY(pick_cfg(L, &cfg));
+    return on_device(device, [&] {
+        if (S == 0) return TRPL_OK;
+        cudaStream_t st = (cudaStream_t)stream;
 
-    KArgs ka;
-    init_kargs(ka, L, tol, max_iter, max_order);
-    ka.x = d_x; ka.ldx = ldx; ka.S = S; ka.pl_stride = 0;
-    ka.sse = d_sse; ka.iters = (long long *)d_iters;
-    ka.mag_col = mag_col; ka.C = C; ka.E = E; ka.plT = 1;
-    ka.flags = flags; ka.pl_dtype = TRPL_F64;
-    for (int c = 0; c < C; c++) {
-        const trpl_curve &src = curves[c];
-        if (!src.d_init || !(src.length > 0)) return TRPL_EINVAL;
-        CurveDev &cv = ka.curves[c];
-        init_curve(cv, src.length, time, L, T, flags, src.d_init);
-        cv.pl_out = nullptr;
-        cv.t_last = 0;
-        for (int e = 0; e < E; e++) {
-            const trpl_obs &o = src.obs[e];
-            if (o.n < 0 || (o.n > 0 && (!o.d_hi || !o.d_whi || !o.d_wlo || !o.d_val)))
-                return TRPL_EINVAL;
-            if (o.n > 0 && (o.hi_max < 1 || o.hi_max > T)) return TRPL_EINVAL;
-            cv.obs[e].n = o.n; cv.obs[e].hi = o.d_hi; cv.obs[e].whi = o.d_whi;
-            cv.obs[e].wlo = o.d_wlo; cv.obs[e].val = o.d_val;
-            if (o.n > 0 && o.hi_max > cv.t_last) cv.t_last = o.hi_max;   // causal truncation
+        KArgs ka;
+        init_kargs(ka, L, tol, max_iter, max_order);
+        ka.x = d_x; ka.ldx = ldx; ka.S = S; ka.pl_stride = 0;
+        ka.sse = d_sse; ka.iters = (long long *)d_iters;
+        ka.mag_col = mag_col; ka.C = C; ka.E = E; ka.plT = 1;
+        ka.flags = flags; ka.pl_dtype = TRPL_F64;
+        for (int c = 0; c < C; c++) {
+            const trpl_curve &src = curves[c];
+            if (!src.d_init || !(src.length > 0)) return TRPL_EINVAL;
+            CurveDev &cv = ka.curves[c];
+            init_curve(cv, src.length, time, L, T, flags, src.d_init);
+            cv.pl_out = nullptr;
+            cv.t_last = 0;
+            for (int e = 0; e < E; e++) {
+                const trpl_obs &o = src.obs[e];
+                if (o.n < 0 || (o.n > 0 && (!o.d_hi || !o.d_whi || !o.d_wlo || !o.d_val)))
+                    return TRPL_EINVAL;
+                if (o.n > 0 && (o.hi_max < 1 || o.hi_max > T)) return TRPL_EINVAL;
+                cv.obs[e].n = o.n; cv.obs[e].hi = o.d_hi; cv.obs[e].whi = o.d_whi;
+                cv.obs[e].wlo = o.d_wlo; cv.obs[e].val = o.d_val;
+                if (o.n > 0 && o.hi_max > cv.t_last) cv.t_last = o.hi_max;   // causal truncation
+            }
         }
-    }
-    Scratch status_cs(st);                     // allocated only after every argument was validated
-    if (d_status) CK(status_cs.alloc(sizeof(int) * (size_t)C * S));
-    ka.status = (int *)status_cs.p;
-    rc = launch_sims(ka, cfg, device, st);
-    if (rc) return rc;
-    const int tb = 256;
-    trpl_finish_kernel<<<(unsigned)((S + tb - 1) / tb), tb, 0, st>>>(d_sse, d_lnl, (const int *)status_cs.p,
-                                                                      d_status, S, C, E);
-    CK(cudaGetLastError());
-    return TRPL_OK;
+        Scratch status_cs(st);                     // allocated only after every argument was validated
+        if (d_status) CK(status_cs.alloc(sizeof(int) * (size_t)C * S));
+        ka.status = (int *)status_cs.p;
+        TRY(launch_sims(ka, cfg, device, st));
+        const int tb = 256;
+        trpl_finish_kernel<<<(unsigned)((S + tb - 1) / tb), tb, 0, st>>>(d_sse, d_lnl, (const int *)status_cs.p,
+                                                                          d_status, S, C, E);
+        CK(cudaGetLastError());
+        return TRPL_OK;
+    });
 }
 
 int trpl_log10_clamp(void *d_pl, int dtype, int64_t n, double min, int device, void *stream)
 {
     if (!d_pl || n < 0 || (dtype != TRPL_F64 && dtype != TRPL_F32)) return TRPL_EINVAL;
-    DeviceGuard guard;
-    int rc = guard.enter(device);
-    if (rc) return rc;
-    if (n == 0) return TRPL_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    int nsm = 0;
-    CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
-    const int tb = 256;
-    long long blocks = (n + tb - 1) / tb;
-    if (blocks > (long long)nsm * 16) blocks = (long long)nsm * 16;
-    if (dtype == TRPL_F64)
-        trpl_log10_kernel_f64<<<(unsigned)blocks, tb, 0, st>>>((double *)d_pl, n, min);
-    else
-        trpl_log10_kernel_f32<<<(unsigned)blocks, tb, 0, st>>>((float *)d_pl, n, min);
-    CK(cudaGetLastError());
-    return TRPL_OK;
+    return on_device(device, [&] {
+        if (n == 0) return TRPL_OK;
+        cudaStream_t st = (cudaStream_t)stream;
+        unsigned grid;
+        TRY(stride_grid(device, n, 256, 16, &grid));
+        if (dtype == TRPL_F64)
+            trpl_log10_kernel<<<grid, 256, 0, st>>>((double *)d_pl, n, min);
+        else
+            trpl_log10_kernel<<<grid, 256, 0, st>>>((float *)d_pl, n, min);
+        CK(cudaGetLastError());
+        return TRPL_OK;
+    });
 }
 
 int trpl_lnp_accumulate(double *d_P, const double *d_pl, int64_t S, int64_t n, int64_t ld,
                         const double *d_values, const double *d_mag, int device, void *stream)
 {
     if (!d_P || !d_pl || !d_values || !d_mag || S < 0 || n < 0 || ld < n) return TRPL_EINVAL;
-    DeviceGuard guard;
-    int rc = guard.enter(device);
-    if (rc) return rc;
-    if (S == 0) return TRPL_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    int nsm = 0;
-    CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
-    const int tb = 256;
-    long long blocks = (S * 32 + tb - 1) / tb;
-    if (blocks > (long long)nsm * 8) blocks = (long long)nsm * 8;
-    trpl_lnp_kernel<<<(unsigned)blocks, tb, 0, st>>>(d_P, d_pl, S, n, ld, d_values, d_mag);
-    CK(cudaGetLastError());
-    return TRPL_OK;
+    return on_device(device, [&] {
+        if (S == 0) return TRPL_OK;
+        unsigned grid;
+        TRY(stride_grid(device, S * 32, 256, 8, &grid));    // one warp per sample
+        trpl_lnp_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_P, d_pl, S, n, ld, d_values, d_mag);
+        CK(cudaGetLastError());
+        return TRPL_OK;
+    });
 }
 
 int trpl_obs_prepare(const double *times, int32_t n, double time, int T, int32_t *hi, double *whi,
@@ -423,69 +441,56 @@ int trpl_obs_prepare(const double *times, int32_t n, double time, int T, int32_t
 int trpl_lse_partial(const double *d_x, int64_t n, double *d_out2, int device, void *stream)
 {
     if (!d_x || !d_out2 || n < 0) return TRPL_EINVAL;
-    DeviceGuard guard;
-    int rc = guard.enter(device);
-    if (rc) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    trpl_lse_init_kernel<<<1, 1, 0, st>>>(d_out2);
-    if (n > 0) {
-        int nsm = 0;
-        CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
-        const int tb = 256;
-        long long blocks = (n + tb - 1) / tb;
-        if (blocks > (long long)nsm * 8) blocks = (long long)nsm * 8;
-        trpl_lse_max_kernel<<<(unsigned)blocks, tb, 0, st>>>(d_x, n, d_out2);
-        trpl_lse_sum_kernel<<<(unsigned)blocks, tb, 0, st>>>(d_x, n, d_out2);
-    }
-    CK(cudaGetLastError());
-    return TRPL_OK;
+    return on_device(device, [&] {
+        cudaStream_t st = (cudaStream_t)stream;
+        trpl_lse_init_kernel<<<1, 1, 0, st>>>(d_out2);
+        if (n > 0) {
+            unsigned grid;
+            TRY(stride_grid(device, n, 256, 8, &grid));
+            trpl_lse_max_kernel<<<grid, 256, 0, st>>>(d_x, n, d_out2);
+            trpl_lse_sum_kernel<<<grid, 256, 0, st>>>(d_x, n, d_out2);
+        }
+        CK(cudaGetLastError());
+        return TRPL_OK;
+    });
 }
-
 
 int trpl_random_grid(double *d_x, int64_t S, int64_t ldx, const double *minx, const double *maxx,
                      const int32_t *do_log, int ncol, int override_flags, uint64_t seed,
                      uint64_t first_sample, int device, void *stream)
 {
     if (!d_x || !minx || !maxx || !do_log || S < 0 || ncol < 1 || ncol > 16 || ldx < ncol) return TRPL_EINVAL;
-    DeviceGuard guard;
-    int rc = guard.enter(device);
-    if (rc) return rc;
-    if (S == 0) return TRPL_OK;
-    GridArgs ga;
-    memset(&ga, 0, sizeof(ga));
-    for (int j = 0; j < ncol; j++) {
-        if (!(minx[j] <= maxx[j]) || (do_log[j] && minx[j] != maxx[j] && !(minx[j] > 0))) return TRPL_EINVAL;
-        ga.lo[j] = minx[j]; ga.hi[j] = maxx[j]; ga.do_log[j] = do_log[j];
-    }
-    ga.ncol = ncol;
-    ga.eq_mu = (override_flags & 1) && ncol > 3;
-    ga.eq_s = (override_flags & 2) && ncol > 6;
-    ga.eq_auger = (override_flags & 4) && ncol > 8;
-    int nsm = 0;
-    CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
-    const int tb = 256;
-    long long blocks = (S * ncol + tb - 1) / tb;
-    if (blocks > (long long)nsm * 16) blocks = (long long)nsm * 16;
-    trpl_random_grid_kernel<<<(unsigned)blocks, tb, 0, (cudaStream_t)stream>>>(d_x, S, ldx, ga, seed, first_sample);
-    CK(cudaGetLastError());
-    return TRPL_OK;
+    return on_device(device, [&] {
+        if (S == 0) return TRPL_OK;
+        GridArgs ga;
+        memset(&ga, 0, sizeof(ga));
+        for (int j = 0; j < ncol; j++) {
+            if (!(minx[j] <= maxx[j]) || (do_log[j] && minx[j] != maxx[j] && !(minx[j] > 0))) return TRPL_EINVAL;
+            ga.lo[j] = minx[j]; ga.hi[j] = maxx[j]; ga.do_log[j] = do_log[j];
+        }
+        ga.ncol = ncol;
+        ga.eq_mu = (override_flags & 1) && ncol > 3;
+        ga.eq_s = (override_flags & 2) && ncol > 6;
+        ga.eq_auger = (override_flags & 4) && ncol > 8;
+        unsigned grid;
+        TRY(stride_grid(device, S * ncol, 256, 16, &grid));
+        trpl_random_grid_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_x, S, ldx, ga, seed, first_sample);
+        CK(cudaGetLastError());
+        return TRPL_OK;
+    });
 }
 
 int trpl_posterior_weights(const double *d_lnp, int64_t n, double lse, double *d_w, int device, void *stream)
 {
     if (!d_lnp || !d_w || n < 0) return TRPL_EINVAL;
-    DeviceGuard guard;
-    int rc = guard.enter(device);
-    if (rc) return rc;
-    if (n == 0) return TRPL_OK;
-    int nsm = 0;
-    CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
-    const int tb = 256;
-    long long blocks = (n + tb - 1) / tb;
-    if (blocks > (long long)nsm * 16) blocks = (long long)nsm * 16;
-    trpl_weights_kernel<<<(unsigned)blocks, tb, 0, (cudaStream_t)stream>>>(d_lnp, n, lse, d_w);
-    CK(cudaGetLastError());
-    return TRPL_OK;
+    return on_device(device, [&] {
+        if (n == 0) return TRPL_OK;
+        unsigned grid;
+        TRY(stride_grid(device, n, 256, 16, &grid));
+        trpl_weights_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_lnp, n, lse, d_w);
+        CK(cudaGetLastError());
+        return TRPL_OK;
+    });
 }
 
 int trpl_weighted_hist(const double *d_x, int64_t n, int64_t ldx, int colx, int coly, const double *d_w,
@@ -497,93 +502,80 @@ int trpl_weighted_hist(const double *d_x, int64_t n, int64_t ldx, int colx, int 
     if (coly >= 0 && (nby < 1 || !(hiy > loy))) return TRPL_EINVAL;
     const long long nb = (long long)nbx * (coly >= 0 ? nby : 1);
     if (nb > 8192) return TRPL_EUNSUPPORTED;
-    DeviceGuard guard;
-    int rc = guard.enter(device);
-    if (rc) return rc;
-    if (n == 0) return TRPL_OK;
-    int nsm = 0;
-    CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
-    const int tb = 256;
-    long long blocks = (n + tb - 1) / tb;
-    if (blocks > (long long)nsm * 4) blocks = (long long)nsm * 4;
-    const size_t smem = (size_t)nb * sizeof(double);
-    CK(cudaFuncSetAttribute((const void *)trpl_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 65536));
-    trpl_hist_kernel<<<(unsigned)blocks, tb, smem, (cudaStream_t)stream>>>(d_x, ldx, colx, coly, d_w, n, lox, hix,
-                                                                            nbx, loy, hiy, nby, d_hist);
-    CK(cudaGetLastError());
-    return TRPL_OK;
+    return on_device(device, [&] {
+        if (n == 0) return TRPL_OK;
+        unsigned grid;
+        TRY(stride_grid(device, n, 256, 4, &grid));
+        const size_t smem = (size_t)nb * sizeof(double);
+        CK(cudaFuncSetAttribute((const void *)trpl_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 65536));
+        trpl_hist_kernel<<<grid, 256, smem, (cudaStream_t)stream>>>(d_x, ldx, colx, coly, d_w, n, lox, hix,
+                                                                    nbx, loy, hiy, nby, d_hist);
+        CK(cudaGetLastError());
+        return TRPL_OK;
+    });
 }
 
 int trpl_weighted_moments(const double *d_x, int64_t n, int64_t ldx, int ncol, const double *d_w,
                           double *d_out, int device, void *stream)
 {
     if (!d_x || !d_w || !d_out || n < 0 || ncol < 1 || ncol > 15 || ldx < ncol) return TRPL_EINVAL;
-    DeviceGuard guard;
-    int rc = guard.enter(device);
-    if (rc) return rc;
-    if (n == 0) return TRPL_OK;
-    int nsm = 0;
-    CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
-    if (ncol == 13 || ncol == 12) {
-        long long nb = (n + 127) / 128;
-        if (nb > (long long)nsm * 2) nb = (long long)nsm * 2;
-        if (ncol == 13)
-            trpl_moments_kernel_fixed<13><<<(unsigned)nb, 128, 0, (cudaStream_t)stream>>>(d_x, ldx, d_w, n, d_out);
-        else
-            trpl_moments_kernel_fixed<12><<<(unsigned)nb, 128, 0, (cudaStream_t)stream>>>(d_x, ldx, d_w, n, d_out);
+    return on_device(device, [&] {
+        if (n == 0) return TRPL_OK;
+        cudaStream_t st = (cudaStream_t)stream;
+        unsigned grid;
+        if (ncol == 13 || ncol == 12) {
+            TRY(stride_grid(device, n, 128, 2, &grid));
+            if (ncol == 13)
+                trpl_moments_kernel_fixed<13><<<grid, 128, 0, st>>>(d_x, ldx, d_w, n, d_out);
+            else
+                trpl_moments_kernel_fixed<12><<<grid, 128, 0, st>>>(d_x, ldx, d_w, n, d_out);
+        } else {
+            TRY(stride_grid(device, n, 256, 8, &grid));
+            const size_t smem = (size_t)(1 + ncol + ncol * ncol) * sizeof(double);
+            trpl_moments_kernel<<<grid, 256, smem, st>>>(d_x, ldx, ncol, d_w, n, d_out);
+        }
         CK(cudaGetLastError());
         return TRPL_OK;
-    }
-    long long blocks = (n + 255) / 256;
-    if (blocks > (long long)nsm * 8) blocks = (long long)nsm * 8;
-    const size_t smem = (size_t)(1 + ncol + ncol * ncol) * sizeof(double);
-    trpl_moments_kernel<<<(unsigned)blocks, 256, smem, (cudaStream_t)stream>>>(d_x, ldx, ncol, d_w, n, d_out);
-    CK(cudaGetLastError());
-    return TRPL_OK;
+    });
 }
 
 int trpl_selftest_rcp(const double *d_x, double *d_y, int64_t n, int device, void *stream)
 {
     if (!d_x || !d_y || n < 0) return TRPL_EINVAL;
-    DeviceGuard guard;
-    int rc = guard.enter(device);
-    if (rc) return rc;
-    if (n == 0) return TRPL_OK;
-    long long blocks = (n + 255) / 256;
-    if (blocks > 4096) blocks = 4096;
-    trpl_rcp_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(d_x, d_y, n);
-    CK(cudaGetLastError());
-    return TRPL_OK;
+    return on_device(device, [&] {
+        if (n == 0) return TRPL_OK;
+        long long blocks = (n + 255) / 256;
+        if (blocks > 4096) blocks = 4096;
+        trpl_rcp_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(d_x, d_y, n);
+        CK(cudaGetLastError());
+        return TRPL_OK;
+    });
 }
 
 int trpl_bench_dfma(int device, int iters, double *tflops, double *ms)
 {
     if (!tflops || iters < 1) return TRPL_EINVAL;
-    DeviceGuard guard;
-    int rc = guard.enter(device);
-    if (rc) return rc;
-    int nsm = 0;
-    CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
-    double *out = nullptr;
-    CK(cudaMalloc((void **)&out, sizeof(double)));
-    const int tb = 256, blocks = nsm * 8;
-    cudaEvent_t e0, e1;
-    CK(cudaEventCreate(&e0));
-    CK(cudaEventCreate(&e1));
-    trpl_dfma_kernel<<<blocks, tb>>>(out, iters / 4 + 1, 1.0);   // warm-up
-    CK(cudaEventRecord(e0));
-    trpl_dfma_kernel<<<blocks, tb>>>(out, iters, 1.0);
-    CK(cudaEventRecord(e1));
-    CK(cudaEventSynchronize(e1));
-    float t = 0.f;
-    CK(cudaEventElapsedTime(&t, e0, e1));
-    const double flop = 2.0 * 8 * 16 * (double)iters * tb * (double)blocks;
-    *tflops = flop / (t * 1e-3) / 1e12;
-    if (ms) *ms = t;
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
-    cudaFree(out);
-    return TRPL_OK;
+    return on_device(device, [&] {
+        int nsm = 0;
+        CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
+        Scratch out(0);                            // legacy default stream, where the kernels run
+        CK(out.alloc(sizeof(double)));
+        const int tb = 256, blocks = nsm * 8;
+        Event e0, e1;
+        CK(e0.create());
+        CK(e1.create());
+        trpl_dfma_kernel<<<blocks, tb>>>((double *)out.p, iters / 4 + 1, 1.0);   // warm-up
+        CK(cudaEventRecord(e0.e));
+        trpl_dfma_kernel<<<blocks, tb>>>((double *)out.p, iters, 1.0);
+        CK(cudaEventRecord(e1.e));
+        CK(cudaEventSynchronize(e1.e));
+        float t = 0.f;
+        CK(cudaEventElapsedTime(&t, e0.e, e1.e));
+        const double flop = 2.0 * 8 * 16 * (double)iters * tb * (double)blocks;
+        *tflops = flop / (t * 1e-3) / 1e12;
+        if (ms) *ms = t;
+        return TRPL_OK;
+    });
 }
 
 }  // extern "C"

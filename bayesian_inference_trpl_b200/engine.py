@@ -6,6 +6,7 @@ Shapes follow the reference: simPar = [Length, Time, L, T, plT, pT, tol, MAX]
 e_data = [(t_list, logPL_list, unc_list)] per observation file (bayes_io.py:99-102).
 """
 import ctypes
+import threading
 import time
 
 import numpy as np
@@ -34,6 +35,12 @@ def _row_stride(t):
 
 def _stream(dev):
     return ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+
+
+def _call(name, dev, *args):
+    """Run export `name` with `args` on `dev` and its current stream (every stream-ordered export takes
+    those two last); raise on a negative return code."""
+    return check(getattr(_lib.lib(), name)(*args, dev.index, _stream(dev)), name)
 
 
 def host_wait(dev=None):
@@ -132,7 +139,6 @@ class Problem:
                     for e in range(e0, e1):
                         self.obs[e][c].fill(curves[c - c0].obs[e - e0])
                 self.parts.append((e0, e1, c0, c1, curves))
-        self.curves = self.parts[0][4]
 
     def steps_per_sample(self):
         """Time steps actually integrated per sample (sum over curves, causal truncation included)."""
@@ -140,7 +146,7 @@ class Problem:
 
 
 _PROBLEMS = {}          # digest -> Problem, insertion-ordered (small LRU)
-_PINNED = {}            # (tag, shape, dtype) -> pinned host staging tensor
+_STAGING = threading.local()   # .bufs: (tag, shape, dtype) -> pinned host staging tensor of one host thread
 
 
 def cached_problem(simPar, iniPar, e_data, device=None, keep=4):
@@ -169,14 +175,18 @@ def cached_problem(simPar, iniPar, e_data, device=None, keep=4):
 
 
 def pinned(tag, shape, dtype):
-    """Reusable pinned host staging buffer."""
+    """Reusable pinned host staging buffer of the calling thread.  Each host thread has its own, so
+    threads that run the same batch shape never write and read one buffer around async copies."""
+    bufs = getattr(_STAGING, "bufs", None)
+    if bufs is None:
+        bufs = _STAGING.bufs = {}
     key = (tag, tuple(shape), dtype)
-    t = _PINNED.get(key)
+    t = bufs.get(key)
     if t is None:
-        if len(_PINNED) > 16:
-            _PINNED.clear()
+        if len(bufs) > 16:
+            bufs.clear()
         t = torch.empty(tuple(shape), dtype=dtype).pin_memory()
-        _PINNED[key] = t
+        bufs[key] = t
     return t
 
 
@@ -193,12 +203,10 @@ def solve_pl(matpar, init, length, time, L, T, plT=1, tol=7, max_iter=10000, out
     status = torch.zeros(S, dtype=torch.int32, device=dev)
     iters = torch.zeros(S, dtype=torch.int64, device=dev) if want_iters else None
     flags = F_INIT_GRID_UNITS if init_grid_units else 0
-    rc = _lib.lib().trpl_solve_pl(
-        _ptr(matpar), S, _row_stride(matpar), _ptr(init), float(length), float(time), int(L), int(T),
-        int(plT), int(tol), int(max_iter), int(max_order), flags, _ptr(pl),
-        F32 if out_dtype == torch.float32 else F64, npl, _ptr(status), _ptr(iters),
-        dev.index, _stream(dev))
-    check(rc, "trpl_solve_pl")
+    _call("trpl_solve_pl", dev,
+          _ptr(matpar), S, _row_stride(matpar), _ptr(init), float(length), float(time), int(L), int(T),
+          int(plT), int(tol), int(max_iter), int(max_order), flags, _ptr(pl),
+          F32 if out_dtype == torch.float32 else F64, npl, _ptr(status), _ptr(iters))
     return pl, status, iters
 
 
@@ -223,12 +231,10 @@ def solve_loglik(X, problem, log_pl=True, self_normalize=False, emulate_f32=Fals
     for e0, e1, c0, c1, curves in problem.parts:
         sse = torch.empty((e1 - e0, c1 - c0, S), dtype=torch.float64, device=dev)
         st = status if len(problem.parts) == 1 else torch.zeros(S, dtype=torch.int32, device=dev)
-        rc = _lib.lib().trpl_solve_loglik(
-            _ptr(X), S, _row_stride(X), mag_col, curves, c1 - c0, e1 - e0, problem.Time, problem.L,
-            problem.T, problem.tol, problem.MAX, int(max_order), flags, _ptr(sse), _ptr(lnl[e0:e1]),
-            _ptr(st), _ptr(iters[c0:c1]) if (iters is not None and e0 == 0) else None, dev.index,
-            _stream(dev))
-        check(rc, "trpl_solve_loglik")
+        _call("trpl_solve_loglik", dev,
+              _ptr(X), S, _row_stride(X), mag_col, curves, c1 - c0, e1 - e0, problem.Time, problem.L,
+              problem.T, problem.tol, problem.MAX, int(max_order), flags, _ptr(sse), _ptr(lnl[e0:e1]),
+              _ptr(st), _ptr(iters[c0:c1]) if (iters is not None and e0 == 0) else None)
         if st is not status:
             status |= st
     return lnl, status, iters
@@ -237,18 +243,15 @@ def solve_loglik(X, problem, log_pl=True, self_normalize=False, emulate_f32=Fals
 def log10_clamp_(t, MIN):
     """probs.fastlog on a device tensor (in place)."""
     assert t.is_cuda and t.is_contiguous() and t.dtype in (torch.float32, torch.float64)
-    rc = _lib.lib().trpl_log10_clamp(_ptr(t), F32 if t.dtype == torch.float32 else F64, t.numel(),
-                                     float(MIN), t.device.index, _stream(t.device))
-    check(rc, "trpl_log10_clamp")
+    _call("trpl_log10_clamp", t.device, _ptr(t), F32 if t.dtype == torch.float32 else F64, t.numel(), float(MIN))
     return t
 
 
 def lnp_accumulate_(P, pl, values, mag):
     """probs.prob on device tensors: P[j] -= sum_i (pl[j,i] + mag[j] - values[i])^2 (in place)."""
     assert P.is_cuda and pl.dtype == torch.float64 and pl.stride(1) == 1
-    rc = _lib.lib().trpl_lnp_accumulate(_ptr(P), _ptr(pl), pl.shape[0], pl.shape[1], pl.stride(0),
-                                        _ptr(values), _ptr(mag), P.device.index, _stream(P.device))
-    check(rc, "trpl_lnp_accumulate")
+    _call("trpl_lnp_accumulate", P.device,
+          _ptr(P), _ptr(pl), pl.shape[0], pl.shape[1], pl.stride(0), _ptr(values), _ptr(mag))
     return P
 
 
@@ -256,8 +259,7 @@ def lse_partial(x):
     """(max, sum exp(x - max)) over the finite entries of a device vector -> tensor [2]."""
     assert x.is_cuda and x.dtype == torch.float64 and x.is_contiguous()
     out = torch.empty(2, dtype=torch.float64, device=x.device)
-    rc = _lib.lib().trpl_lse_partial(_ptr(x), x.numel(), _ptr(out), x.device.index, _stream(x.device))
-    check(rc, "trpl_lse_partial")
+    _call("trpl_lse_partial", x.device, _ptr(x), x.numel(), _ptr(out))
     return out
 
 
@@ -284,11 +286,9 @@ def random_grid_device(minX, maxX, do_log, num_points, seed, first_sample=0, ove
     dl = np.ascontiguousarray(do_log, dtype=np.int32)
     ncol = lo.shape[0]
     X = out if out is not None else torch.empty((num_points, ncol), dtype=torch.float64, device=dev)
-    rc = _lib.lib().trpl_random_grid(_ptr(X), num_points, X.stride(0) if num_points > 1 else ncol,
-                                     lo.ctypes.data_as(ctypes.c_void_p), hi.ctypes.data_as(ctypes.c_void_p),
-                                     dl.ctypes.data_as(ctypes.c_void_p), ncol, int(override_flags),
-                                     int(seed), int(first_sample), dev.index, _stream(dev))
-    check(rc, "trpl_random_grid")
+    _call("trpl_random_grid", dev, _ptr(X), num_points, _row_stride(X),
+          lo.ctypes.data_as(ctypes.c_void_p), hi.ctypes.data_as(ctypes.c_void_p),
+          dl.ctypes.data_as(ctypes.c_void_p), ncol, int(override_flags), int(seed), int(first_sample))
     return X
 
 
@@ -296,8 +296,7 @@ def posterior_weights(lnp, lse):
     """w = exp(lnP - lse) on the device (NaN -> 0)."""
     assert lnp.is_cuda and lnp.dtype == torch.float64 and lnp.is_contiguous()
     w = torch.empty_like(lnp)
-    check(_lib.lib().trpl_posterior_weights(_ptr(lnp), lnp.numel(), float(lse), _ptr(w),
-                                            lnp.device.index, _stream(lnp.device)), "trpl_posterior_weights")
+    _call("trpl_posterior_weights", lnp.device, _ptr(lnp), lnp.numel(), float(lse), _ptr(w))
     return w
 
 
@@ -306,9 +305,8 @@ def weighted_hist(X, colx, w, lox, hix, nbx, coly=-1, loy=0.0, hiy=1.0, nby=1, o
     assert X.is_cuda and X.dtype == torch.float64 and X.stride(1) == 1
     shape = (nbx,) if coly < 0 else (nbx, nby)
     h = out if out is not None else torch.zeros(shape, dtype=torch.float64, device=X.device)
-    check(_lib.lib().trpl_weighted_hist(_ptr(X), X.shape[0], _row_stride(X), int(colx), int(coly), _ptr(w),
-                                        float(lox), float(hix), int(nbx), float(loy), float(hiy), int(nby),
-                                        _ptr(h), X.device.index, _stream(X.device)), "trpl_weighted_hist")
+    _call("trpl_weighted_hist", X.device, _ptr(X), X.shape[0], _row_stride(X), int(colx), int(coly), _ptr(w),
+          float(lox), float(hix), int(nbx), float(loy), float(hiy), int(nby), _ptr(h))
     return h
 
 
@@ -317,6 +315,5 @@ def weighted_moments(X, w, ncol=None, out=None):
     assert X.is_cuda and X.dtype == torch.float64 and X.stride(1) == 1
     ncol = X.shape[1] if ncol is None else ncol
     o = out if out is not None else torch.zeros(1 + ncol + ncol * ncol, dtype=torch.float64, device=X.device)
-    check(_lib.lib().trpl_weighted_moments(_ptr(X), X.shape[0], _row_stride(X), int(ncol), _ptr(w), _ptr(o),
-                                           X.device.index, _stream(X.device)), "trpl_weighted_moments")
+    _call("trpl_weighted_moments", X.device, _ptr(X), X.shape[0], _row_stride(X), int(ncol), _ptr(w), _ptr(o))
     return o
