@@ -172,18 +172,19 @@ def rank_and_world():
     return 0, None
 
 
-def _bayes_philox(N, num_exp, minX, maxX, do_log, init_params, sim_params, e_data, sim_flags, gpu_info, logger):
+def _bayes_philox(N, num_exp, minX, maxX, do_log, init_params, sim_params, e_data, sim_flags, gpu_info, logger,
+                  exchange=None):
     """sim_flags["sampler"] == "philox": every rank draws ONLY its own contiguous rows of the sample
     matrix on its GPU (counter-based Philox4x32-10, `first_sample` = first row of the shard, so the
     shards of any world size concatenate to the single-rank draw bit for bit), runs the fused path on
     them and the tables are all-gathered once at the end.  X never crosses PCIe on the way in; the
     bounds arrive already in engine units (parallel_bayes_gpu.py:183-184), so the unit conversion is
-    part of the draw."""
-    import torch.distributed as dist
+    part of the draw.  `exchange` (default: distributed.TorchExchange) supplies the rank and the gather."""
     from . import distributed
+    ex = exchange if exchange is not None else distributed.TorchExchange()
     dev = engine.require_cuda(gpu_info.get("device", None))
     S = int(sim_flags["num_points"])
-    rank, world = (dist.get_rank(), dist.get_world_size()) if dist.is_initialized() else (0, 1)
+    rank, world = ex.rank_world()
     lo, hi = distributed.shard_bounds(S, rank, world)
     flags = ((1 if sim_flags["override_equal_mu"] else 0) | (2 if sim_flags["override_equal_s"] else 0)
              | (4 if sim_flags["override_equal_auger"] else 0))
@@ -196,20 +197,20 @@ def _bayes_philox(N, num_exp, minX, maxX, do_log, init_params, sim_params, e_dat
     bad = int((status != 0).sum().item())
     if bad and logger is not None:
         logger.warning("%d samples did not converge (lnL = NaN for them)", bad)
-    P = distributed.gather_rows(lnl, S)
-    X = distributed.gather_rows(Xd.t().contiguous(), S).t()
+    P = ex.gather_rows(lnl, S)
+    X = ex.gather_rows(Xd.t().contiguous(), S).t()
     return np.arange(S), P.cpu().numpy(), np.ascontiguousarray(X.cpu().numpy())
 
 
 def bayes(model, N, P, minX, maxX, do_log, init_params, sim_params, e_data, sim_flags, gpu_info,
-          logger=None):
+          logger=None, exchange=None):
     """Draw the sample matrix, evaluate this rank's share of the likelihood table, return
     (N, P, X) like bayeslib.bayes (bayeslib.py:207-252).  Columns of P that belong to other ranks
     stay 0 exactly as in the reference (bayes_io.py:134) -- except with sim_flags["sampler"] ==
-    "philox", where the complete table comes back on every rank."""
+    "philox", where the complete table comes back on every rank (gathered through `exchange`)."""
     if sim_flags.get("sampler", "numpy") == "philox":
         return _bayes_philox(N, len(e_data), minX, maxX, do_log, init_params, sim_params, e_data,
-                             sim_flags, gpu_info, logger)
+                             sim_flags, gpu_info, logger, exchange=exchange)
     num_gpus = gpu_info["num_gpus"]
     solver_time = np.zeros(num_gpus)
     err_sq_time = np.zeros(num_gpus)

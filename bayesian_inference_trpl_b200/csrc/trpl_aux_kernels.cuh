@@ -182,13 +182,13 @@ __global__ void trpl_random_grid_kernel(double *x, long long S, long long ldx, c
 }
 
 // ---- posterior products (Visualization/utils.py:157-285) -------------------------------------
+__device__ __forceinline__ double posterior_weight(double v, double lse) { return (v == v) ? exp(v - lse) : 0.0; }
+
 __global__ void trpl_weights_kernel(const double *lnp, long long n, double lse, double *w)
 {
     const long long stride = (long long)gridDim.x * blockDim.x;
-    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += stride) {
-        const double v = lnp[i];
-        w[i] = (v == v) ? exp(v - lse) : 0.0;
-    }
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += stride)
+        w[i] = posterior_weight(lnp[i], lse);
 }
 
 // numpy.histogram bin of v over nb uniform bins on [lo, hi] (right edge inclusive), or -1

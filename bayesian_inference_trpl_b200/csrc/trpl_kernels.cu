@@ -1,7 +1,7 @@
 // trpl_kernels.cu -- sm_100a kernels + C ABI of libtrpl_b200.so (see include/trpl_b200.h).
 //
 // Files: trpl_solver.cuh (hot path), trpl_aux_kernels.cuh (small kernels), trpl_common.cuh (argument
-// structs, helpers), this file (host side + C ABI).
+// structs, helpers), trpl_host.cuh (host helpers shared with trpl_nccl.cu), this file (host side + C ABI).
 //
 // Hot path replaced: pvSimPCR.py:14-401 (tEvol/iterate/pcreduce/norm2 + pvSim host driver) and
 // probs.py:20-85 (kernel_lnP, log_kernel), plus the glue bayeslib.simulate runs between them
@@ -36,6 +36,7 @@
 #include "trpl_common.cuh"
 #include "trpl_solver.cuh"
 #include "trpl_aux_kernels.cuh"
+#include "trpl_host.cuh"
 
 using namespace trpl;
 
@@ -44,24 +45,6 @@ namespace {
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
-thread_local char g_cuda_err[256] = "";
-
-int cuda_fail(cudaError_t e, const char *what)
-{
-    snprintf(g_cuda_err, sizeof(g_cuda_err), "%s: %s", what, cudaGetErrorString(e));
-    return TRPL_ECUDA;
-}
-#define CK(call)                                                   \
-    do {                                                           \
-        cudaError_t e_ = (call);                                   \
-        if (e_ != cudaSuccess) return cuda_fail(e_, #call);        \
-    } while (0)
-// propagates a TRPL_E* code of a host helper
-#define TRY(call)                                                  \
-    do {                                                           \
-        if (int rc_ = (call)) return rc_;                          \
-    } while (0)
-
 // pvSimPCR.py:327-331 (same expression order; pow() is glibc's, as in CPython)
 void make_scales(double length, double time, int L, int T, double *sc, double *dx_o, double *dt_o)
 {
@@ -74,17 +57,6 @@ void make_scales(double length, double time, int L, int T, double *sc, double *d
     *dx_o = dx; *dt_o = dt;
 }
 
-// stream-ordered device scratch, released on every exit path
-struct Scratch {
-    void *p = nullptr;
-    cudaStream_t st;
-    explicit Scratch(cudaStream_t s) : st(s) {}
-    cudaError_t alloc(size_t bytes) { return cudaMallocAsync(&p, bytes, st); }
-    ~Scratch() { if (p) cudaFreeAsync(p, st); }
-    Scratch(const Scratch &) = delete;
-    Scratch &operator=(const Scratch &) = delete;
-};
-
 // CUDA event, destroyed on every exit path
 struct Event {
     cudaEvent_t e = nullptr;
@@ -94,18 +66,6 @@ struct Event {
     Event(const Event &) = delete;
     Event &operator=(const Event &) = delete;
 };
-
-// Grid of a grid-stride kernel over `work` items with `tb` threads per block: one item per thread, at most
-// `per_sm` blocks per SM of `device`.  The reductions accumulate one partial sum per block, so their grouping
-// (and last bits) follow this grid.
-int stride_grid(int device, long long work, int tb, int per_sm, unsigned *grid)
-{
-    int nsm = 0;
-    CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
-    const long long want = (work + tb - 1) / tb, cap = (long long)nsm * per_sm;
-    *grid = (unsigned)(want < cap ? want : cap);
-    return TRPL_OK;
-}
 
 struct Cfg { int M; bool pad; int W; };      // W = warps per simulation (1: warp kernel, >1: CTA kernel)
 int pick_cfg(int L, Cfg *cfg)
@@ -205,38 +165,6 @@ void init_curve(CurveDev &cv, double length, double time, int L, int T, int flag
     cv.init_mul = (flags & TRPL_F_INIT_GRID_UNITS) ? 1.0 : cv.scales[0];
     cv.redim = pow(dx, 2.0) * dt;
     cv.init = d_init;
-}
-
-// Makes `device` current for the duration of one C-ABI call and restores the caller's device on every
-// exit path (torch reads its current device from the runtime; a library must not change it).
-struct DeviceGuard {
-    int prev = -1;
-    bool switched = false;
-    int enter(int device)
-    {
-        int n = 0;
-        if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0 || device < 0 || device >= n) {
-            cudaGetLastError();
-            return TRPL_ENODEVICE;
-        }
-        CK(cudaGetDevice(&prev));
-        if (prev != device) {
-            CK(cudaSetDevice(device));
-            switched = true;
-        }
-        return TRPL_OK;
-    }
-    ~DeviceGuard() { if (switched) cudaSetDevice(prev); }
-};
-
-// Runs `work` (returning a TRPL_* code) with `device` current, or returns why the device cannot be entered.
-// Entry points validate their arguments before this and call it once, so every one has the same shape.
-template <class F>
-int on_device(int device, F &&work)
-{
-    DeviceGuard guard;
-    TRY(guard.enter(device));
-    return work();
 }
 
 int launch_sims(KArgs &ka, const Cfg &cfg, int device, cudaStream_t st)

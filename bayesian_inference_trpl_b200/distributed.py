@@ -60,3 +60,23 @@ def merge_block_cyclic(P_local):
         t = t.cuda()
     dist.all_reduce(t, op=dist.ReduceOp.SUM)
     return t
+
+
+class TorchExchange:
+    """The exchange points of a run (parallel_bayes_gpu.run) over torch.distributed, or none on a single
+    rank: the default.  nccl.Communicator offers the same methods over the C ABI, without a process group."""
+
+    def rank_world(self):
+        return (dist.get_rank(), dist.get_world_size()) if dist.is_initialized() else (0, 1)
+
+    def gather_rows(self, local, n_total):
+        return gather_rows(local, n_total)
+
+    def merge_block_cyclic(self, P_local):
+        return merge_block_cyclic(P_local)
+
+    def posterior_weights_full(self, lnP):
+        """Weights of a full table [S] on the device, normalised on this rank."""
+        from . import engine
+        ms = engine.lse_partial(lnP)
+        return normalize_posterior(lnP, ms[0] + torch.log(ms[1]))

@@ -48,22 +48,36 @@ def default_config():
 
 
 def run(init_filename, experimental_data_filename, out_filename, cfg=None, seed=42, logger=None,
-        posterior=False):
+        posterior=False, exchange=None, nccl_id_file=None):
     """Same sequence as the reference `__main__` block; returns (P, X in common units).
 
     Launchers: (a) torchrun, one rank per GPU: the per-rank tables are merged over NCCL and rank 0
     exports; (b) SLURM array tasks like the reference (no communication): task k fills its
     block-cyclic columns and EVERY task exports, into `<out>_task<k>` when there is more than one
     task, with NaN in the columns it does not own (`merge_task_exports` joins them afterwards);
-    the task count must agree with gpu_info["num_gpus"]."""
+    the task count must agree with gpu_info["num_gpus"].
+
+    `exchange` selects how the ranks of (a) exchange results: None or "torch" (torch.distributed, a
+    process group over NCCL); "cabi" (an nccl.Communicator over the C ABI, no process group; a
+    multi-rank run bootstraps it through the file `nccl_id_file`); or an object with the methods of
+    distributed.TorchExchange, such as an open nccl.Communicator whose rank and size match
+    RANK/WORLD_SIZE.  SLURM array tasks are not co-scheduled and always merge through files."""
     import torch
     import torch.distributed as dist
     cfg = cfg or default_config()
     rank, world = bayeslib.rank_and_world()
     slurm = os.getenv("SLURM_ARRAY_TASK_ID") is not None
-    if not slurm and world is not None and world > 1 and not dist.is_initialized():
-        torch.cuda.set_device(int(os.environ.get("LOCAL_RANK", rank)))
-        dist.init_process_group("nccl")
+    if exchange == "cabi":
+        with _cabi_communicator(rank, world, slurm, nccl_id_file) as comm:
+            return run(init_filename, experimental_data_filename, out_filename, cfg=cfg, seed=seed, logger=logger,
+                       posterior=posterior, exchange=comm)
+    if exchange is None or exchange == "torch":
+        if not slurm and world is not None and world > 1 and not dist.is_initialized():
+            torch.cuda.set_device(int(os.environ.get("LOCAL_RANK", rank)))
+            dist.init_process_group("nccl")
+        exchange = distributed.TorchExchange()
+    elif isinstance(exchange, str):
+        raise ValueError("exchange must be 'torch', 'cabi' or an exchange object, not %r" % exchange)
     np.random.seed(seed)
     simPar = [cfg["Length"], cfg["Time"], cfg["L"], cfg["T"], cfg["plT"], cfg["pT"], cfg["tol"], cfg["MAX"]]
     ic_flags, sim_flags, gpu_info = cfg["ic_flags"], dict(cfg["sim_flags"]), dict(cfg["gpu_info"])
@@ -97,10 +111,10 @@ def run(init_filename, experimental_data_filename, out_filename, cfg=None, seed=
     maxX *= unit_conversions
     clock0 = perf_counter()
     N, P, X = bayeslib.bayes(pvSim, np.array([0]), None, minX, maxX, do_log, iniPar, simPar, e_data,
-                             sim_flags, gpu_info, logger=logger)
+                             sim_flags, gpu_info, logger=logger, exchange=exchange)
     complete = sim_flags.get("sampler", "numpy") == "philox"
     if not complete and not slurm and world and world > 1:
-        P = np.asarray(distributed.merge_block_cyclic(P).cpu())
+        P = np.asarray(exchange.merge_block_cyclic(P).cpu())
     if logger is not None:
         logger.info("Bayesim took %.3f s", perf_counter() - clock0)
     X = X / unit_conversions
@@ -109,17 +123,33 @@ def run(init_filename, experimental_data_filename, out_filename, cfg=None, seed=
         mine = bayeslib.owned_columns(P.shape[1], gpu_info, rank)
         P = np.where(mine[None, :], P, np.nan)             # 0 would read as the best possible likelihood
         outs = ["%s_task%d" % (of.rstrip("/\\"), rank) for of in outs]
+    if posterior:                                          # on every rank: the exchange may be collective
+        W = [exchange.posterior_weights_full(torch.from_numpy(np.nan_to_num(P[i], nan=-np.inf)).cuda()).cpu().numpy()
+             for i in range(len(outs))]
     if slurm or rank == 0:
         for i, of in enumerate(outs):
             bayes_io.export(of, P[i], X, logger=logger)
             if posterior:
-                t = torch.from_numpy(np.nan_to_num(P[i], nan=-np.inf)).cuda()
-                from . import engine
-                ms = engine.lse_partial(t)
-                lse = ms[0] + torch.log(ms[1])
-                w = distributed.normalize_posterior(t, lse).cpu().numpy()
-                np.save(os.path.join(of, os.path.basename(os.path.normpath(of)) + "_BAYRAN_W.npy"), w)
+                np.save(os.path.join(of, os.path.basename(os.path.normpath(of)) + "_BAYRAN_W.npy"), W[i])
     return P, X
+
+
+def _cabi_communicator(rank, world, slurm, nccl_id_file):
+    """nccl.Communicator of this rank for run(..., exchange="cabi"): rank and size from RANK/WORLD_SIZE, the
+    GPU from LOCAL_RANK, like torchrun; a single process needs no id file."""
+    import torch
+    from . import nccl
+    if slurm:
+        raise RuntimeError("SLURM array tasks are not co-scheduled, so NCCL cannot join them: they merge "
+                           "through files (merge_task_exports)")
+    if world is None or world == 1:
+        return nccl.Communicator(nccl.unique_id(), 0, 1, torch.cuda.current_device())
+    if not nccl_id_file:
+        raise ValueError("exchange='cabi' with %d ranks needs an id file every rank can read (--nccl-id-file)"
+                         % world)
+    device = int(os.environ.get("LOCAL_RANK", rank))
+    torch.cuda.set_device(device)
+    return nccl.Communicator.from_file(nccl_id_file, rank, world, device)
 
 
 def merge_task_exports(out_filename, num_tasks):
@@ -151,6 +181,12 @@ def main(argv=None):
                     help="numpy: the reference's host draw (np.random.seed(42), bit-compatible); philox: every rank "
                          "draws only its own rows on its GPU")
     ap.add_argument("--sims-per-gpu", type=int, default=None)
+    ap.add_argument("--exchange", choices=["torch", "cabi"], default="torch",
+                    help="how torchrun ranks exchange results: torch.distributed, or the NCCL C ABI "
+                         "(libtrpl_b200_nccl.so) without a process group")
+    ap.add_argument("--nccl-id-file", default=None,
+                    help="with --exchange cabi and several ranks: a path every rank can read, which must not "
+                         "exist yet; rank 0 writes the communicator id there")
     args = ap.parse_args(argv)
     logging.basicConfig(level=logging.INFO, format="%(asctime)s %(levelname)s: %(message)s")
     logger = logging.getLogger("Bayes Logger Main")
@@ -169,7 +205,8 @@ def main(argv=None):
         cfg["ic_flags"]["time_cutoff"] = args.final_time
     outs = [args.out] if len(args.observations) == 1 else \
         [args.out + "_%d" % i for i in range(len(args.observations))]
-    run(args.excitations, args.observations, outs, cfg=cfg, logger=logger, posterior=args.posterior)
+    run(args.excitations, args.observations, outs, cfg=cfg, logger=logger, posterior=args.posterior,
+        exchange=args.exchange, nccl_id_file=args.nccl_id_file)
 
 
 if __name__ == "__main__":
