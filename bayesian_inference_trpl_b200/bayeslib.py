@@ -172,6 +172,12 @@ def rank_and_world():
     return 0, None
 
 
+def override_flags(sim_flags):
+    """Bit mask of the override_equal_* flags for the device samplers (1: mu, 2: s, 4: auger)."""
+    return ((1 if sim_flags["override_equal_mu"] else 0) | (2 if sim_flags["override_equal_s"] else 0)
+            | (4 if sim_flags["override_equal_auger"] else 0))
+
+
 def _bayes_philox(N, num_exp, minX, maxX, do_log, init_params, sim_params, e_data, sim_flags, gpu_info, logger,
                   exchange=None):
     """sim_flags["sampler"] == "philox": every rank draws ONLY its own contiguous rows of the sample
@@ -186,10 +192,8 @@ def _bayes_philox(N, num_exp, minX, maxX, do_log, init_params, sim_params, e_dat
     S = int(sim_flags["num_points"])
     rank, world = ex.rank_world()
     lo, hi = distributed.shard_bounds(S, rank, world)
-    flags = ((1 if sim_flags["override_equal_mu"] else 0) | (2 if sim_flags["override_equal_s"] else 0)
-             | (4 if sim_flags["override_equal_auger"] else 0))
     Xd = engine.random_grid_device(minX, maxX, do_log, hi - lo, int(sim_flags.get("seed", 42)),
-                                   first_sample=lo, override_flags=flags, device=dev.index)
+                                   first_sample=lo, override_flags=override_flags(sim_flags), device=dev.index)
     problem = engine.cached_problem(list(sim_params), init_params, e_data, device=dev.index)
     lnl, status, _ = engine.solve_loglik(Xd, problem, log_pl=sim_flags["log_pl"],
                                          self_normalize=sim_flags["self_normalize"],

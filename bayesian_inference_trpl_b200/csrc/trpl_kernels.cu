@@ -36,7 +36,9 @@
 #include "trpl_common.cuh"
 #include "trpl_solver.cuh"
 #include "trpl_aux_kernels.cuh"
+#include "trpl_ensemble.cuh"
 #include "trpl_host.cuh"
+#include "trpl_b200_ensemble.h"
 
 using namespace trpl;
 
@@ -191,6 +193,38 @@ int launch_sims(KArgs &ka, const Cfg &cfg, int device, cudaStream_t st)
         CK(cudaGetLastError());
     }
     return TRPL_OK;
+}
+
+// Sample bounds of trpl_random_grid and the ensemble sampler: log columns need minx > 0 unless fixed.
+int grid_args(const double *minx, const double *maxx, const int32_t *do_log, int ncol, int override_flags,
+              GridArgs *ga)
+{
+    memset(ga, 0, sizeof(*ga));
+    for (int j = 0; j < ncol; j++) {
+        if (!(minx[j] <= maxx[j]) || (do_log[j] && minx[j] != maxx[j] && !(minx[j] > 0))) return TRPL_EINVAL;
+        ga->lo[j] = minx[j]; ga->hi[j] = maxx[j]; ga->do_log[j] = do_log[j];
+    }
+    ga->ncol = ncol;
+    ga->eq_mu = (override_flags & 1) && ncol > 3;
+    ga->eq_s = (override_flags & 2) && ncol > 6;
+    ga->eq_auger = (override_flags & 4) && ncol > 8;
+    return TRPL_OK;
+}
+
+// Free columns of the ensemble sampler: not fixed (minx == maxx) and not an override target.
+int free_columns(const GridArgs &ga)
+{
+    int d = 0;
+    for (int j = 0; j < ga.ncol; j++)
+        d += ga.lo[j] != ga.hi[j] && !(ga.eq_mu && j == 2) && !(ga.eq_s && j == 6) && !(ga.eq_auger && j == 8);
+    return d;
+}
+
+// The n walkers [first, first + n) lie in one half of an even ensemble of W >= 2.
+bool one_half(int64_t n, int64_t first, int64_t W)
+{
+    const int64_t h = W / 2;
+    return W >= 2 && W % 2 == 0 && n >= 0 && first >= 0 && (first + n <= h || (first >= h && first + n <= W));
 }
 
 }  // namespace
@@ -391,15 +425,7 @@ int trpl_random_grid(double *d_x, int64_t S, int64_t ldx, const double *minx, co
     return on_device(device, [&] {
         if (S == 0) return TRPL_OK;
         GridArgs ga;
-        memset(&ga, 0, sizeof(ga));
-        for (int j = 0; j < ncol; j++) {
-            if (!(minx[j] <= maxx[j]) || (do_log[j] && minx[j] != maxx[j] && !(minx[j] > 0))) return TRPL_EINVAL;
-            ga.lo[j] = minx[j]; ga.hi[j] = maxx[j]; ga.do_log[j] = do_log[j];
-        }
-        ga.ncol = ncol;
-        ga.eq_mu = (override_flags & 1) && ncol > 3;
-        ga.eq_s = (override_flags & 2) && ncol > 6;
-        ga.eq_auger = (override_flags & 4) && ncol > 8;
+        TRY(grid_args(minx, maxx, do_log, ncol, override_flags, &ga));
         unsigned grid;
         TRY(stride_grid(device, S * ncol, 256, 16, &grid));
         trpl_random_grid_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_x, S, ldx, ga, seed, first_sample);
@@ -502,6 +528,51 @@ int trpl_bench_dfma(int device, int iters, double *tflops, double *ms)
         const double flop = 2.0 * 8 * 16 * (double)iters * tb * (double)blocks;
         *tflops = flop / (t * 1e-3) / 1e12;
         if (ms) *ms = t;
+        return TRPL_OK;
+    });
+}
+
+// ---- ensemble sampler (include/trpl_b200_ensemble.h) ------------------------------------------------------
+int trpl_stretch_propose(const double *d_x, int64_t n, int64_t ldx, int64_t first_walker, int64_t n_walkers,
+                         const double *d_comp, int64_t ld_comp, const double *minx, const double *maxx,
+                         const int32_t *do_log, int ncol, int override_flags, double a, uint64_t seed,
+                         uint32_t step, double *d_y, int64_t ldy, double *d_logq, int device, void *stream)
+{
+    if (!d_x || !d_comp || !minx || !maxx || !do_log || !d_y || !d_logq || ncol < 1 || ncol > 16 ||
+        ldx < ncol || ldy < ncol || !(a > 1) || !one_half(n, first_walker, n_walkers) || ld_comp < n_walkers / 2)
+        return TRPL_EINVAL;
+    GridArgs ga;
+    TRY(grid_args(minx, maxx, do_log, ncol, override_flags, &ga));
+    const int d = free_columns(ga);
+    if (n_walkers < 2 * (d > 1 ? d : 1)) return TRPL_EINVAL;
+    return on_device(device, [&] {
+        if (n == 0) return TRPL_OK;
+        unsigned grid;
+        TRY(stride_grid(device, n, 128, 8, &grid));
+        trpl_stretch_propose_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(d_x, n, ldx, first_walker, d_comp, ld_comp,
+                                                                            n_walkers / 2, ga, d, a, seed, step, d_y,
+                                                                            ldy, d_logq);
+        CK(cudaGetLastError());
+        return TRPL_OK;
+    });
+}
+
+int trpl_stretch_accept(double *d_x, int64_t n, int64_t ldx, int64_t first_walker, int64_t n_walkers, int ncol,
+                        double *d_lnl, const double *d_y, int64_t ldy, const double *d_lnl_y,
+                        const double *d_logq, double temperature, uint64_t seed, uint32_t step,
+                        int32_t *d_accepted, int device, void *stream)
+{
+    if (!d_x || !d_lnl || !d_y || !d_lnl_y || !d_logq || ncol < 1 || ncol > 16 || ldx < ncol || ldy < ncol ||
+        !(temperature > 0) || !one_half(n, first_walker, n_walkers))
+        return TRPL_EINVAL;
+    return on_device(device, [&] {
+        if (n == 0) return TRPL_OK;
+        unsigned grid;
+        TRY(stride_grid(device, n, 128, 8, &grid));
+        trpl_stretch_accept_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(d_x, n, ldx, first_walker, ncol, d_lnl, d_y,
+                                                                           ldy, d_lnl_y, d_logq, temperature, seed,
+                                                                           step, d_accepted);
+        CK(cudaGetLastError());
         return TRPL_OK;
     });
 }

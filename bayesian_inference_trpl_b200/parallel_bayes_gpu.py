@@ -9,7 +9,11 @@ implemented command line (`README.md:4,29`: OBS EXC OUT) actually parsed.
 Every rank draws the same sample matrix (global seed 42, parallel_bayes_gpu.py:35), evaluates
 its block-cyclic share on its GPU with the fused kernel, the likelihood tables are merged over
 NCCL and rank 0 writes <OUT>_BAYRAN_P.npy / _BAYRAN_X.npy (plus the normalised posterior
-weights when --posterior is given)."""
+weights when --posterior is given).
+
+With --sampler ensemble the posterior of ONE observation file is sampled by an ensemble MCMC instead
+(stretch moves, ensemble.py): rank 0 writes the chain, <OUT>_MCMC_X.npy [steps+1, walkers, 13] in common
+units and <OUT>_MCMC_P.npy [steps+1, walkers] (the untempered lnL)."""
 import argparse
 import logging
 import os
@@ -43,7 +47,8 @@ def default_config():
         "gpu_info": {"sims_per_gpu": 2 ** 10, "num_gpus": 1},
         "sim_flags": {"load_PL_from_file": False, "override_equal_auger": False,
                       "override_equal_mu": False, "override_equal_s": False, "log_pl": True,
-                      "self_normalize": False, "random_sample": True, "num_points": 2 ** 17},
+                      "self_normalize": False, "random_sample": True, "num_points": 2 ** 17,
+                      "walkers": 1024, "steps": 100, "temperature": 1.0},
     }
 
 
@@ -61,10 +66,18 @@ def run(init_filename, experimental_data_filename, out_filename, cfg=None, seed=
     process group over NCCL); "cabi" (an nccl.Communicator over the C ABI, no process group; a
     multi-rank run bootstraps it through the file `nccl_id_file`); or an object with the methods of
     distributed.TorchExchange, such as an open nccl.Communicator whose rank and size match
-    RANK/WORLD_SIZE.  SLURM array tasks are not co-scheduled and always merge through files."""
+    RANK/WORLD_SIZE.  SLURM array tasks are not co-scheduled and always merge through files.
+
+    cfg["sim_flags"]["sampler"] == "ensemble" samples the posterior of the one observation file with
+    cfg["sim_flags"]["walkers"] walkers for ["steps"] steps at ["temperature"] (ensemble.sample) and returns
+    (lnL chain [steps+1, W], X chain [steps+1, W, 13] in common units)."""
     import torch
     import torch.distributed as dist
     cfg = cfg or default_config()
+    ensemble = cfg["sim_flags"].get("sampler", "numpy") == "ensemble"
+    if ensemble and len(experimental_data_filename) != 1:
+        raise ValueError("the ensemble sampler samples the posterior of one observation file; got %d (run one "
+                         "ensemble per file)" % len(experimental_data_filename))
     rank, world = bayeslib.rank_and_world()
     slurm = os.getenv("SLURM_ARRAY_TASK_ID") is not None
     if exchange == "cabi":
@@ -104,11 +117,17 @@ def run(init_filename, experimental_data_filename, out_filename, cfg=None, seed=
             raise RuntimeError("SLURM_ARRAY_TASK_ID=%d but gpu_info['num_gpus']=%d" % (rank, gpu_info["num_gpus"]))
         if sim_flags.get("sampler", "numpy") == "philox" and gpu_info["num_gpus"] > 1:
             raise RuntimeError("the philox sampler shards over torch.distributed ranks; use torchrun")
+        if ensemble:
+            raise RuntimeError("the ensemble sampler exchanges walkers every step, which SLURM array tasks "
+                               "cannot do; use torchrun")
     elif world is not None:
         gpu_info["num_gpus"] = world
 
     minX *= unit_conversions
     maxX *= unit_conversions
+    if ensemble:
+        return _run_ensemble(iniPar, simPar, e_data, minX, maxX, do_log, sim_flags, gpu_info, out_filename[0],
+                             exchange, logger)
     clock0 = perf_counter()
     N, P, X = bayeslib.bayes(pvSim, np.array([0]), None, minX, maxX, do_log, iniPar, simPar, e_data,
                              sim_flags, gpu_info, logger=logger, exchange=exchange)
@@ -131,6 +150,36 @@ def run(init_filename, experimental_data_filename, out_filename, cfg=None, seed=
             bayes_io.export(of, P[i], X, logger=logger)
             if posterior:
                 np.save(os.path.join(of, os.path.basename(os.path.normpath(of)) + "_BAYRAN_W.npy"), W[i])
+    return P, X
+
+
+def _run_ensemble(iniPar, simPar, e_data, minX, maxX, do_log, sim_flags, gpu_info, out, exchange, logger):
+    """run() with sampler "ensemble": bounds in engine units; rank 0 writes <out>_MCMC_[XP].npy."""
+    from . import engine, ensemble
+    rank, world = exchange.rank_world()
+    dev = engine.require_cuda(gpu_info.get("device", None))
+    W, steps, seed = int(sim_flags["walkers"]), int(sim_flags["steps"]), int(sim_flags["seed"])
+    flags = bayeslib.override_flags(sim_flags)
+    X0 = ensemble.initial_walkers(W, minX, maxX, do_log, seed, flags, rank, world, device=dev.index)
+    problem = engine.cached_problem(list(simPar), iniPar, e_data, device=dev.index)
+    loglik = ensemble.solver_loglik(problem, log_pl=sim_flags["log_pl"], self_normalize=sim_flags["self_normalize"],
+                                    emulate_f32=gpu_info.get("emulate_f32", False))
+    clock0 = perf_counter()
+    chain = ensemble.sample(X0, loglik, minX, maxX, do_log, steps, n_walkers=W, override_flags=flags,
+                            temperature=float(sim_flags["temperature"]), seed=seed, exchange=exchange)
+    P, X = chain.lnl.cpu().numpy(), chain.X.cpu().numpy() / unit_conversions
+    acc = chain.acceptance.cpu().numpy()
+    if logger is not None:
+        logger.info("ensemble: %d walkers x %d steps on %d rank(s) took %.3f s; acceptance fraction %.3f overall, "
+                    "%.3f over the last half", W, steps, world, perf_counter() - clock0,
+                    acc.mean() if steps else float("nan"), acc[steps // 2:].mean() if steps else float("nan"))
+    if rank == 0:
+        os.makedirs(out, exist_ok=True)
+        base = os.path.basename(os.path.normpath(out))
+        np.save(os.path.join(out, base + "_MCMC_X.npy"), X)
+        np.save(os.path.join(out, base + "_MCMC_P.npy"), P)
+        if logger is not None:
+            logger.info("wrote %s_MCMC_[XP].npy to %s", base, out)
     return P, X
 
 
@@ -177,9 +226,14 @@ def main(argv=None):
     ap.add_argument("--time-steps", type=int, default=None)
     ap.add_argument("--final-time", type=float, default=None)
     ap.add_argument("--posterior", action="store_true", help="also write normalised posterior weights")
-    ap.add_argument("--sampler", choices=["numpy", "philox"], default="numpy",
+    ap.add_argument("--sampler", choices=["numpy", "philox", "ensemble"], default="numpy",
                     help="numpy: the reference's host draw (np.random.seed(42), bit-compatible); philox: every rank "
-                         "draws only its own rows on its GPU")
+                         "draws only its own rows on its GPU; ensemble: MCMC with stretch moves (one observation "
+                         "file), writes the chain to <out>_MCMC_X.npy / _MCMC_P.npy")
+    ap.add_argument("--walkers", type=int, default=None, help="ensemble: number of walkers (even)")
+    ap.add_argument("--steps", type=int, default=None, help="ensemble: number of steps")
+    ap.add_argument("--temperature", type=float, default=None,
+                    help="ensemble: sample exp(lnL / temperature) (default 1)")
     ap.add_argument("--sims-per-gpu", type=int, default=None)
     ap.add_argument("--exchange", choices=["torch", "cabi"], default="torch",
                     help="how torchrun ranks exchange results: torch.distributed, or the NCCL C ABI "
@@ -194,6 +248,9 @@ def main(argv=None):
     if args.num_points:
         cfg["sim_flags"]["num_points"] = args.num_points
     cfg["sim_flags"]["sampler"] = args.sampler
+    for key in ("walkers", "steps", "temperature"):
+        if getattr(args, key) is not None:
+            cfg["sim_flags"][key] = getattr(args, key)
     if args.sims_per_gpu:
         cfg["gpu_info"]["sims_per_gpu"] = args.sims_per_gpu
     if args.length:
