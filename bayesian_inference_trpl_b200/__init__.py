@@ -8,7 +8,7 @@ HagesLab/Bayesian-Inference-TRPL.  Python surface mirrors the reference:
     engine.solve_loglik           fused device-resident path (no reference counterpart)
 """
 from . import _lib, bayes_io, bayes_validate, bayeslib, distributed, engine, probs, pvsim  # noqa: F401
-from . import ensemble, parallel_bayes_gpu, posterior  # noqa: F401
+from . import ensemble, parallel_bayes_gpu, posterior, tempering  # noqa: F401
 from ._lib import TrplError, build  # noqa: F401
 from .probs import fastlog, prob  # noqa: F401
 from .pvsim import pvSim  # noqa: F401

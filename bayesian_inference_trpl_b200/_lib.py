@@ -68,7 +68,7 @@ EXPORTS = list(_SIGNATURES)
 def build(force=False, verbose=False):
     """Compile csrc/trpl_kernels.cu into libtrpl_b200.so for sm_100a (cross-compiles without a GPU)."""
     csrc = os.path.dirname(SRC)
-    deps = [os.path.join(INCLUDE, h) for h in ("trpl_b200.h", "trpl_b200_ensemble.h")] + [
+    deps = [os.path.join(INCLUDE, h) for h in ("trpl_b200.h", "trpl_b200_ensemble.h", "trpl_b200_tempering.h")] + [
         os.path.join(csrc, f) for f in os.listdir(csrc) if f.endswith((".cu", ".cuh"))]
     if (not force and os.path.exists(LIB_PATH)
             and os.path.getmtime(LIB_PATH) >= max(os.path.getmtime(d) for d in deps)):

@@ -39,6 +39,7 @@
 #include "trpl_ensemble.cuh"
 #include "trpl_host.cuh"
 #include "trpl_b200_ensemble.h"
+#include "trpl_b200_tempering.h"
 
 using namespace trpl;
 
@@ -225,6 +226,21 @@ bool one_half(int64_t n, int64_t first, int64_t W)
 {
     const int64_t h = W / 2;
     return W >= 2 && W % 2 == 0 && n >= 0 && first >= 0 && (first + n <= h || (first >= h && first + n <= W));
+}
+
+// A ladder of include/trpl_b200_tempering.h: 1 <= K <= TRPL_MAX_RUNGS, T_0 > 0, strictly increasing, and
+// only the last entry may be +inf.
+bool ladder(const double *temperatures, int K, Ladder *lad)
+{
+    if (!temperatures || K < 1 || K > TRPL_MAX_RUNGS) return false;
+    memset(lad, 0, sizeof(*lad));
+    for (int t = 0; t < K; t++) {
+        const double T = temperatures[t];
+        if (!(t == 0 ? T > 0 : T > temperatures[t - 1]) || (T == INFINITY && t != K - 1)) return false;
+        lad->t[t] = T;
+    }
+    lad->k = K;
+    return true;
 }
 
 }  // namespace
@@ -532,14 +548,35 @@ int trpl_bench_dfma(int device, int iters, double *tflops, double *ms)
     });
 }
 
-// ---- ensemble sampler (include/trpl_b200_ensemble.h) ------------------------------------------------------
+// ---- ensemble sampler (include/trpl_b200_ensemble.h): one rung of the tempered entries --------------------
 int trpl_stretch_propose(const double *d_x, int64_t n, int64_t ldx, int64_t first_walker, int64_t n_walkers,
                          const double *d_comp, int64_t ld_comp, const double *minx, const double *maxx,
                          const int32_t *do_log, int ncol, int override_flags, double a, uint64_t seed,
                          uint32_t step, double *d_y, int64_t ldy, double *d_logq, int device, void *stream)
 {
+    return trpl_tempered_propose(d_x, n, ldx, first_walker, n_walkers, 1, d_comp, ld_comp, minx, maxx, do_log, ncol,
+                                 override_flags, a, seed, step, d_y, ldy, d_logq, device, stream);
+}
+
+int trpl_stretch_accept(double *d_x, int64_t n, int64_t ldx, int64_t first_walker, int64_t n_walkers, int ncol,
+                        double *d_lnl, const double *d_y, int64_t ldy, const double *d_lnl_y,
+                        const double *d_logq, double temperature, uint64_t seed, uint32_t step,
+                        int32_t *d_accepted, int device, void *stream)
+{
+    return trpl_tempered_accept(d_x, n, ldx, first_walker, n_walkers, 1, &temperature, ncol, d_lnl, d_y, ldy,
+                                d_lnl_y, d_logq, seed, step, d_accepted, device, stream);
+}
+
+// ---- parallel tempering (include/trpl_b200_tempering.h) --------------------------------------------------
+int trpl_tempered_propose(const double *d_x, int64_t n, int64_t ldx, int64_t first_walker, int64_t n_walkers,
+                          int n_rungs, const double *d_comp, int64_t ld_comp, const double *minx,
+                          const double *maxx, const int32_t *do_log, int ncol, int override_flags, double a,
+                          uint64_t seed, uint32_t step, double *d_y, int64_t ldy, double *d_logq, int device,
+                          void *stream)
+{
     if (!d_x || !d_comp || !minx || !maxx || !do_log || !d_y || !d_logq || ncol < 1 || ncol > 16 ||
-        ldx < ncol || ldy < ncol || !(a > 1) || !one_half(n, first_walker, n_walkers) || ld_comp < n_walkers / 2)
+        ldx < ncol || ldy < ncol || !(a > 1) || !one_half(n, first_walker, n_walkers) || ld_comp < n_walkers / 2 ||
+        n_rungs < 1 || n_rungs > TRPL_MAX_RUNGS)
         return TRPL_EINVAL;
     GridArgs ga;
     TRY(grid_args(minx, maxx, do_log, ncol, override_flags, &ga));
@@ -549,29 +586,49 @@ int trpl_stretch_propose(const double *d_x, int64_t n, int64_t ldx, int64_t firs
         if (n == 0) return TRPL_OK;
         unsigned grid;
         TRY(stride_grid(device, n, 128, 8, &grid));
-        trpl_stretch_propose_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(d_x, n, ldx, first_walker, d_comp, ld_comp,
-                                                                            n_walkers / 2, ga, d, a, seed, step, d_y,
-                                                                            ldy, d_logq);
+        trpl_stretch_propose_kernel<<<dim3(grid, n_rungs), 128, 0, (cudaStream_t)stream>>>(
+            d_x, n, ldx, first_walker, n_walkers, d_comp, ld_comp, n_walkers / 2, ga, d, a, seed, step, d_y, ldy,
+            d_logq);
         CK(cudaGetLastError());
         return TRPL_OK;
     });
 }
 
-int trpl_stretch_accept(double *d_x, int64_t n, int64_t ldx, int64_t first_walker, int64_t n_walkers, int ncol,
-                        double *d_lnl, const double *d_y, int64_t ldy, const double *d_lnl_y,
-                        const double *d_logq, double temperature, uint64_t seed, uint32_t step,
-                        int32_t *d_accepted, int device, void *stream)
+int trpl_tempered_accept(double *d_x, int64_t n, int64_t ldx, int64_t first_walker, int64_t n_walkers,
+                         int n_rungs, const double *temperatures, int ncol, double *d_lnl, const double *d_y,
+                         int64_t ldy, const double *d_lnl_y, const double *d_logq, uint64_t seed, uint32_t step,
+                         int32_t *d_accepted, int device, void *stream)
 {
+    Ladder lad;
     if (!d_x || !d_lnl || !d_y || !d_lnl_y || !d_logq || ncol < 1 || ncol > 16 || ldx < ncol || ldy < ncol ||
-        !(temperature > 0) || !one_half(n, first_walker, n_walkers))
+        !ladder(temperatures, n_rungs, &lad) || !one_half(n, first_walker, n_walkers))
         return TRPL_EINVAL;
     return on_device(device, [&] {
         if (n == 0) return TRPL_OK;
         unsigned grid;
         TRY(stride_grid(device, n, 128, 8, &grid));
-        trpl_stretch_accept_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(d_x, n, ldx, first_walker, ncol, d_lnl, d_y,
-                                                                           ldy, d_lnl_y, d_logq, temperature, seed,
-                                                                           step, d_accepted);
+        trpl_stretch_accept_kernel<<<dim3(grid, n_rungs), 128, 0, (cudaStream_t)stream>>>(
+            d_x, n, ldx, first_walker, n_walkers, ncol, d_lnl, d_y, ldy, d_lnl_y, d_logq, lad, seed, step,
+            d_accepted);
+        CK(cudaGetLastError());
+        return TRPL_OK;
+    });
+}
+
+int trpl_tempered_swap(double *d_x, int64_t n, int64_t ldx, int64_t first_walker, int64_t n_walkers, int n_rungs,
+                       const double *temperatures, int ncol, double *d_lnl, uint64_t seed, uint32_t step,
+                       int32_t *d_swapped, int device, void *stream)
+{
+    Ladder lad;
+    if (!d_x || !d_lnl || ncol < 1 || ncol > 16 || ldx < ncol || !ladder(temperatures, n_rungs, &lad) ||
+        !one_half(n, first_walker, n_walkers))
+        return TRPL_EINVAL;
+    return on_device(device, [&] {
+        if (n == 0 || n_rungs == 1) return TRPL_OK;
+        unsigned grid;
+        TRY(stride_grid(device, n, 128, 8, &grid));
+        trpl_tempered_swap_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(d_x, n, ldx, first_walker, n_walkers, ncol,
+                                                                          d_lnl, lad, seed, step, d_swapped);
         CK(cudaGetLastError());
         return TRPL_OK;
     });

@@ -13,8 +13,12 @@ weights when --posterior is given).
 
 With --sampler ensemble the posterior of ONE observation file is sampled by an ensemble MCMC instead
 (stretch moves, ensemble.py): rank 0 writes the chain, <OUT>_MCMC_X.npy [steps+1, walkers, 13] in common
-units and <OUT>_MCMC_P.npy [steps+1, walkers] (the untempered lnL)."""
+units and <OUT>_MCMC_P.npy [steps+1, walkers] (the untempered lnL).  With --ladder T0 T1 ... [inf] the
+ensemble runs parallel tempering on that ladder (tempering.py): the two files hold the cold rung, and rank 0
+also writes <OUT>_MCMC_PT_P.npy [steps+1, rungs, walkers] and <OUT>_MCMC_PT.json (per-rung mean lnL,
+acceptance, swap acceptance, log-evidence)."""
 import argparse
+import json
 import logging
 import os
 import sys
@@ -70,7 +74,8 @@ def run(init_filename, experimental_data_filename, out_filename, cfg=None, seed=
 
     cfg["sim_flags"]["sampler"] == "ensemble" samples the posterior of the one observation file with
     cfg["sim_flags"]["walkers"] walkers for ["steps"] steps at ["temperature"] (ensemble.sample) and returns
-    (lnL chain [steps+1, W], X chain [steps+1, W, 13] in common units)."""
+    (lnL chain [steps+1, W], X chain [steps+1, W, 13] in common units).  A ladder in
+    cfg["sim_flags"]["ladder"] runs tempering.sample on it instead and returns the cold rung's chains."""
     import torch
     import torch.distributed as dist
     cfg = cfg or default_config()
@@ -78,6 +83,14 @@ def run(init_filename, experimental_data_filename, out_filename, cfg=None, seed=
     if ensemble and len(experimental_data_filename) != 1:
         raise ValueError("the ensemble sampler samples the posterior of one observation file; got %d (run one "
                          "ensemble per file)" % len(experimental_data_filename))
+    if cfg["sim_flags"].get("ladder") is not None:
+        if not ensemble:
+            raise ValueError("a temperature ladder needs the ensemble sampler")
+        if float(cfg["sim_flags"].get("temperature", 1.0)) != 1.0:
+            raise ValueError("a temperature ladder and a sampling temperature exclude each other: the ladder's "
+                             "first entry is the sampled temperature")
+        from . import tempering
+        tempering.check_ladder(cfg["sim_flags"]["ladder"])
     rank, world = bayeslib.rank_and_world()
     slurm = os.getenv("SLURM_ARRAY_TASK_ID") is not None
     if exchange == "cabi":
@@ -160,10 +173,13 @@ def _run_ensemble(iniPar, simPar, e_data, minX, maxX, do_log, sim_flags, gpu_inf
     dev = engine.require_cuda(gpu_info.get("device", None))
     W, steps, seed = int(sim_flags["walkers"]), int(sim_flags["steps"]), int(sim_flags["seed"])
     flags = bayeslib.override_flags(sim_flags)
-    X0 = ensemble.initial_walkers(W, minX, maxX, do_log, seed, flags, rank, world, device=dev.index)
     problem = engine.cached_problem(list(simPar), iniPar, e_data, device=dev.index)
     loglik = ensemble.solver_loglik(problem, log_pl=sim_flags["log_pl"], self_normalize=sim_flags["self_normalize"],
                                     emulate_f32=gpu_info.get("emulate_f32", False))
+    if sim_flags.get("ladder") is not None:
+        return _run_tempered(loglik, minX, maxX, do_log, W, steps, seed, flags, sim_flags["ladder"], dev, out,
+                             exchange, logger)
+    X0 = ensemble.initial_walkers(W, minX, maxX, do_log, seed, flags, rank, world, device=dev.index)
     clock0 = perf_counter()
     chain = ensemble.sample(X0, loglik, minX, maxX, do_log, steps, n_walkers=W, override_flags=flags,
                             temperature=float(sim_flags["temperature"]), seed=seed, exchange=exchange)
@@ -181,6 +197,48 @@ def _run_ensemble(iniPar, simPar, e_data, minX, maxX, do_log, sim_flags, gpu_inf
         if logger is not None:
             logger.info("wrote %s_MCMC_[XP].npy to %s", base, out)
     return P, X
+
+
+def _run_tempered(loglik, minX, maxX, do_log, W, steps, seed, flags, ladder, dev, out, exchange, logger):
+    """_run_ensemble on a temperature ladder: rank 0 writes the cold rung to <out>_MCMC_[XP].npy, every rung's
+    lnL to <out>_MCMC_PT_P.npy and the summary (log-evidence over the second half) to <out>_MCMC_PT.json."""
+    from . import tempering
+    rank, world = exchange.rank_world()
+    T = tempering.check_ladder(ladder)
+    K = T.shape[0]
+    X0 = tempering.initial_walkers(W, K, minX, maxX, do_log, seed, flags, rank, world, device=dev.index)
+    clock0 = perf_counter()
+    chain = tempering.sample(X0, loglik, minX, maxX, do_log, steps, T, n_walkers=W, override_flags=flags, seed=seed,
+                             exchange=exchange)
+    PT, X = chain.lnl.cpu().numpy(), chain.X.cpu().numpy() / unit_conversions
+    acc, swp = chain.acceptance.cpu().numpy(), chain.swap_acceptance.cpu().numpy()
+    burn = steps // 2
+    ev = tempering.log_evidence(PT, T, burn)
+    if logger is not None:
+        logger.info("tempered ensemble: %d rungs x %d walkers x %d steps on %d rank(s) took %.3f s; ln Z = %.6g "
+                    "+- %.3g", K, W, steps, world, perf_counter() - clock0, ev.lnZ, ev.err)
+    if rank == 0:
+        os.makedirs(out, exist_ok=True)
+        base = os.path.join(out, os.path.basename(os.path.normpath(out)))
+        np.save(base + "_MCMC_X.npy", X)
+        np.save(base + "_MCMC_P.npy", PT[:, 0])
+        np.save(base + "_MCMC_PT_P.npy", PT)
+
+        def num(v):
+            return [num(u) for u in v] if np.ndim(v) else (float(v) if np.isfinite(v) else str(float(v)))
+        summary = {"temperatures": num(T), "walkers": W, "steps": steps, "burn": burn,
+                   "mean_lnl": num(ev.mean_lnl),
+                   "acceptance": num(acc[burn:].mean(axis=0) if steps else np.full(K, np.nan)),
+                   "swap_acceptance": num(swp[burn:].mean(axis=0) if steps else np.full(K - 1, np.nan)),
+                   "log_evidence": num(ev.lnZ), "log_evidence_err": num(ev.err),
+                   "beta_min_extrapolated": ev.extrapolated, "prior_rung": bool(np.isinf(T[-1])),
+                   "nonfinite_lnl": int((~np.isfinite(PT)).sum())}
+        with open(base + "_MCMC_PT.json", "w") as fh:
+            json.dump(summary, fh, indent=1)
+        if logger is not None:
+            logger.info("wrote %s_MCMC_[XP].npy, _MCMC_PT_P.npy and _MCMC_PT.json to %s", os.path.basename(base),
+                        out)
+    return PT[:, 0], X
 
 
 def _cabi_communicator(rank, world, slurm, nccl_id_file):
@@ -234,6 +292,10 @@ def main(argv=None):
     ap.add_argument("--steps", type=int, default=None, help="ensemble: number of steps")
     ap.add_argument("--temperature", type=float, default=None,
                     help="ensemble: sample exp(lnL / temperature) (default 1)")
+    ap.add_argument("--ladder", type=float, nargs="+", default=None, metavar="T",
+                    help="ensemble: parallel tempering on these temperatures (strictly increasing from T0 > 0, the "
+                         "last may be inf = the prior); writes the cold rung as without it, plus "
+                         "<out>_MCMC_PT_P.npy and <out>_MCMC_PT.json with the log-evidence")
     ap.add_argument("--sims-per-gpu", type=int, default=None)
     ap.add_argument("--exchange", choices=["torch", "cabi"], default="torch",
                     help="how torchrun ranks exchange results: torch.distributed, or the NCCL C ABI "
@@ -251,6 +313,17 @@ def main(argv=None):
     for key in ("walkers", "steps", "temperature"):
         if getattr(args, key) is not None:
             cfg["sim_flags"][key] = getattr(args, key)
+    if args.ladder is not None:
+        from . import tempering
+        if args.sampler != "ensemble":
+            ap.error("--ladder needs --sampler ensemble")
+        if args.temperature is not None:
+            ap.error("--ladder and --temperature exclude each other: the ladder's first entry is the sampled "
+                     "temperature")
+        try:
+            cfg["sim_flags"]["ladder"] = list(tempering.check_ladder(args.ladder))
+        except ValueError as e:
+            ap.error("--ladder: %s" % e)
     if args.sims_per_gpu:
         cfg["gpu_info"]["sims_per_gpu"] = args.sims_per_gpu
     if args.length:
